@@ -2,7 +2,7 @@
 """bench.py — GraphPOPE geodesic embedding generation on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload flickr-shape]
-                    [--no-cpu-baseline] [--no-secondary]
+                    [--no-cpu-baseline] [--no-secondary] [--dump-outputs DIR]
 
 A *step* is one full pass of the hot path over one synthetic graph already resident in HBM:
 device CSR build (dedup) -> multi-source BFS (persistent kernel) -> fused normalise + concat
@@ -21,6 +21,9 @@ Prints ONE JSON line (rank 0).  Besides the headline (BASELINE config C2) the li
     strong-scaled) — each checked against its oracle, and the cold one-shot cost of the drop-in call.
 `--impl reference` times the reference algorithm (utils.py:64-114: N*K networkx shortest_path calls in a process
 pool) restated in oracle/ on a bounded row sample.
+`--dump-outputs DIR` writes the [N, F+K] float32 matrix of the last timed step to DIR/features.npy (a fixed row sample
+when the whole matrix exceeds DUMP_BYTES).  Inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 from __future__ import annotations
 
@@ -41,6 +44,25 @@ import numpy as np
 METRIC = "anchor-BFS GTEPS (K*|E|/s), geodesic GraphPOPE embedding, Flickr-shape K=256 per GPU"
 UNIT = "GTEPS"
 K_PER_GPU = 256
+DUMP_BYTES = 60_000_000  # --dump-outputs stays below 64 MB
+
+
+def dump_rows(n, cols):
+    """Rows of the [n, cols] float32 matrix that --dump-outputs writes: all of them when they fit in DUMP_BYTES, else
+    a fixed sample (seed 0, ascending)."""
+    rows = min(n, DUMP_BYTES // (4 * max(1, cols)))
+    if rows == n:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, rows, replace=False))
+
+
+def dump_outputs(out_d, directory):
+    import torch
+    idx = dump_rows(*out_d.shape)
+    if idx.size < out_d.size(0):
+        out_d = out_d[torch.as_tensor(idx, device=out_d.device)]
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "features.npy"), out_d.cpu().numpy())
 
 
 # --------------------------------------------------------------------------- CPU reference legs
@@ -549,7 +571,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--secondary", default="c3,c4,c5,cold", help="comma list of secondary lines to run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the [N, F+K] matrix of the last timed step to DIR/features.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours: the reference arm times a row sample and keeps no output")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -691,6 +719,8 @@ def main():
 
     # ---- parity of what the timed loop produced (untimed)
     parity_ok, parity_info = check_device_result(out_d, x_d, ei, n, f, anchors, world, rank, dist)
+    if args.dump_outputs and rank == 0:  # every rank holds the whole matrix (checksums compared above)
+        dump_outputs(out_d, args.dump_outputs)
 
     # ---- stage times: a second pass over the same step with CUDA-event nodes inside the replayed graph (csr build |
     # MS-BFS kernel | epilogue).  An event-record node costs ~4 us of the step, so the timed loop above runs without
@@ -740,7 +770,7 @@ def main():
     for _ in range(3):
         e2e_step()
     barrier()
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
     t0 = time.perf_counter()
     for _ in range(e2e_steps):
         e2e_step()

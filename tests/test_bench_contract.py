@@ -5,6 +5,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
@@ -51,3 +54,48 @@ def test_a_failing_secondary_line_is_reported_not_fatal(capsys):
     res, ok = bench.guarded(boom, 7)
     assert ok is False and res["parity_checked"] is False and "simulated) 7" in res["error"]
     assert bench.guarded(lambda a, b: ({"v": a + b}, True), 1, 2) == ({"v": 3}, True)
+
+
+def test_dump_outputs_row_sample_and_argument_checks():
+    import bench
+
+    rows = bench.dump_rows(89250, 756)  # headline matrix, 270 MB: a fixed row sample under 64 MB
+    assert 4 * 756 * rows.size <= bench.DUMP_BYTES < 64_000_000 and rows.size > 19_000
+    assert np.all(np.diff(rows) > 0) and rows[-1] < 89250
+    assert np.array_equal(rows, bench.dump_rows(89250, 756))
+    assert np.array_equal(bench.dump_rows(1000, 756), np.arange(1000))
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True,
+                           timeout=300, env=env, cwd=ROOT)
+        assert r.returncode == 2 and "error:" in r.stderr, extra
+
+
+@pytest.mark.gpu
+def test_dump_outputs_holds_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs: the row sample of the headline [N, F+K] matrix, x in columns [0, F) and the features
+    bit-equal to the C oracle."""
+    import torch
+
+    import bench
+    from graphpope_b200 import synth
+    from oracle import cbfs
+
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1",
+                        "--no-cpu-baseline", "--no-secondary", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])["steps"] == 2
+    assert sorted(os.listdir(tmp_path)) == ["features.npy"]
+    got = np.load(tmp_path / "features.npy")
+    shape = synth.FLICKR_SHAPE
+    n, f = shape.num_nodes, shape.num_features
+    rows = bench.dump_rows(n, f + bench.K_PER_GPU)
+    assert got.dtype == np.float32 and got.shape == (rows.size, f + bench.K_PER_GPU)
+    assert os.path.getsize(tmp_path / "features.npy") <= 64_000_000
+    x = torch.randn(n, f, device="cuda", generator=torch.Generator("cuda").manual_seed(1)).cpu().numpy()
+    assert np.array_equal(got[:, :f], x[rows])
+    ei = synth.make_graph(shape)
+    anchors = synth.stochastic_anchors(n, bench.K_PER_GPU, 42)
+    want = cbfs.normalise(cbfs.bfs_hops(cbfs.InCsr(ei, n), anchors))[rows]
+    assert np.array_equal(got[:, f:].view(np.uint32), want.view(np.uint32))
