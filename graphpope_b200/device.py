@@ -288,6 +288,146 @@ class GeodesicEngine:
         return out
 
 
+class FeatureStore:
+    """The ``[N, F + K]`` matrix of ``concat_into_features`` (utils.py:129-135) held compactly on the device: x as
+    is, the anchor block as a reached bit plus ``bit_length(max hop)`` hop-bit planes per entry (the format is
+    documented in include/graphpope_b200.h, gp_fstore_*).  Rows are produced on demand by a fused gather kernel, so
+    ``store[n_id]`` stands in for ``data.x[n_id]`` of the trainer (main.py:120,177) without the dense matrix.
+
+    ``FeatureStore(bfs, x)`` packs the last run of an :class:`MsBfs` (the store does not refer to it afterwards).
+    """
+
+    def __init__(self, bfs: MsBfs, x: torch.Tensor | None = None):
+        self._lib = _lib.require_cuda()
+        n, k = bfs.csr.num_nodes, bfs.num_anchors
+        if x is not None:
+            if x.dtype != torch.float32 or x.dim() != 2 or x.size(0) != n:
+                raise TypeError("x must be a float32 tensor of shape [N, F]")
+            x = x.to(device="cuda").contiguous()
+        self.stats = bfs.stats()  # syncs; surfaces index errors of the run
+        planes, words = c_int32(), c_int64()
+        check(self._lib.gp_fstore_layout(bfs._h, byref(planes), byref(words), _stream()))
+        self._raw = torch.empty((n, planes.value, words.value), dtype=torch.uint64, device="cuda")
+        check(self._lib.gp_fstore_pack(bfs._h, _ptr(self._raw), planes.value, _stream()))
+        self._x = x
+        self.num_nodes, self.num_anchors = n, k
+        self.num_features = 0 if x is None else x.size(1)
+        self._bad = torch.zeros(1, dtype=torch.int32, device="cuda")
+
+    @classmethod
+    def build(cls, edge_index, num_nodes: int, anchors, x: torch.Tensor | None = None,
+              symmetrize: bool = False) -> "FeatureStore":
+        """csr build + MS-BFS + pack; the BFS workspace is freed before returning."""
+        ei = torch.as_tensor(edge_index).to(device="cuda", dtype=torch.int64)
+        if ei.dim() != 2 or ei.size(0) != 2:
+            raise ValueError("edge_index must have shape [2, E]")
+        a = torch.as_tensor(np.asarray(anchors, dtype=np.int64).reshape(-1)).cuda()
+        csr = DeviceCsr(int(num_nodes), ei.size(1), symmetrize).build(ei)
+        bfs = MsBfs(csr, max(1, a.numel()))
+        try:
+            return cls(bfs.run(a), x)
+        finally:
+            bfs.close()
+            csr.close()
+
+    # ---- tensor-like surface
+    @property
+    def shape(self) -> torch.Size:
+        return torch.Size((self.num_nodes, self.num_features + self.num_anchors))
+
+    def size(self, dim: int | None = None):
+        return self.shape if dim is None else self.shape[dim]
+
+    @property
+    def dtype(self) -> torch.dtype:
+        return torch.float32
+
+    @property
+    def device(self) -> torch.device:
+        return self._raw.device
+
+    def __len__(self) -> int:
+        return self.num_nodes
+
+    @property
+    def num_planes(self) -> int:
+        return self._raw.size(1)
+
+    @property
+    def nbytes(self) -> int:
+        """Bytes of the anchor block (x is held as given)."""
+        return self._raw.numel() * 8
+
+    @property
+    def raw(self) -> torch.Tensor:
+        """The packed records, uint64 ``[N, P, W]``."""
+        return self._raw
+
+    def gather(self, rows: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
+        """Rows ``rows`` (cuda integer ids; negative ids wrap once) as a cuda float32 ``[B, F + K]``; no host sync.
+        Ids outside ``[-N, N)`` give zero rows and are reported by :meth:`check`."""
+        if not rows.is_cuda or rows.dtype == torch.bool or rows.is_floating_point() or rows.is_complex():
+            raise TypeError("rows must be a cuda integer tensor")
+        rows = rows.reshape(-1).to(torch.int64).contiguous()
+        b, f, k = rows.numel(), self.num_features, self.num_anchors
+        if out is None:
+            out = torch.empty((b, f + k), dtype=torch.float32, device="cuda")
+        elif (not out.is_cuda or out.dtype != torch.float32 or out.dim() != 2 or tuple(out.shape) != (b, f + k)
+              or (out.stride(1) != 1 and f + k > 1)):
+            raise TypeError(f"out must be a cuda float32 [{b}, {f + k}] tensor with unit column stride")
+        x = self._x
+        check(self._lib.gp_fstore_gather(_ptr(self._raw), self.num_nodes, k, self.num_planes, _ptr(rows), b,
+                                         _ptr(x), f, x.stride(0) if x is not None else 0, _ptr(out),
+                                         out.stride(0) if b > 1 else f + k, f, _ptr(self._bad), _stream()))
+        return out
+
+    def check(self):
+        """Syncs.  Raises ``IndexError`` if gathers since the last check met ids outside ``[-N, N)`` (once; the
+        counter is reset)."""
+        bad = int(self._bad.item())
+        if bad:
+            self._bad.zero_()
+            raise IndexError(f"{bad} gathered row ids were outside [-{self.num_nodes}, {self.num_nodes})")
+
+    def __getitem__(self, index):
+        """``store[i]``, ``store[a:b:s]``, ``store[ids]`` with ``ids`` a CPU or cuda integer tensor, a numpy array or
+        a list, with torch's result shapes.  A host-side index is range-checked before anything is launched."""
+        n = self.num_nodes
+        if isinstance(index, tuple):
+            raise TypeError("FeatureStore takes one row index (no tuples)")
+        if isinstance(index, slice):
+            return self.gather(torch.arange(*index.indices(n), device="cuda"))
+        if isinstance(index, (int, np.integer)) and not isinstance(index, (bool, np.bool_)):
+            index = int(index)
+            if not -n <= index < n:
+                raise IndexError(f"index {index} is out of bounds for dimension 0 with size {n}")
+            return self.gather(torch.tensor([index], device="cuda"))[0]
+        if not torch.is_tensor(index):
+            if isinstance(index, (bool, np.bool_)):
+                raise TypeError("FeatureStore does not take boolean masks")
+            index = torch.as_tensor(np.asarray(index))
+            if index.numel() == 0:
+                index = index.to(torch.int64)  # [] -> an empty batch, as in torch
+        if index.dtype == torch.bool:
+            raise TypeError("FeatureStore does not take boolean masks")
+        if index.is_floating_point() or index.is_complex():
+            raise IndexError("tensors used as indices must be integer tensors")
+        if not index.is_cuda:
+            if index.numel() and (int(index.min()) < -n or int(index.max()) >= n):
+                bad = index[(index < -n) | (index >= n)].reshape(-1)[0]
+                raise IndexError(f"index {int(bad)} is out of bounds for dimension 0 with size {n}")
+            index = index.to("cuda")
+        return self.gather(index).reshape(*index.shape, self.num_features + self.num_anchors)
+
+    def to_dense(self) -> torch.Tensor:
+        """The dense cuda float32 ``[N, F + K]`` matrix (what ``GRAPHPOPE_OUTPUT=cuda`` returns)."""
+        return self.gather(torch.arange(self.num_nodes, device="cuda"))
+
+    def __repr__(self):
+        return (f"FeatureStore(shape={tuple(self.shape)}, num_planes={self.num_planes}, "
+                f"nbytes={self.nbytes}, device={self.device})")
+
+
 def normalize_into(dist_u16: torch.Tensor, out: torch.Tensor, col_offset: int = 0) -> torch.Tensor:
     lib = _lib.require_cuda()
     n, k = dist_u16.shape

@@ -54,7 +54,10 @@ VERBOSE = os.environ.get("GRAPHPOPE_QUIET", "0") != "1"
 def _output_device() -> str:
     """``GRAPHPOPE_OUTPUT=cuda`` keeps the ``[N, F+K]`` matrix in HBM (SURVEY §8f rank 3: the trainer's
     ``x[n_id]`` gathers, main.py:120,177, then run on the device and the 91 MB device->host copy plus the
-    host concat disappear).  Default ``cpu`` = the reference's contract."""
+    host concat disappear).  ``GRAPHPOPE_OUTPUT=compact`` returns a :class:`device.FeatureStore` instead: x on the
+    device plus the anchor block in ``1 + bit_length(max hop)`` bits per entry, whose ``store[n_id]`` gathers the
+    trainer's rows without ever forming the dense matrix (geodesic space only; node2vec values have no compact form
+    and behave as ``cuda``).  Default ``cpu`` = the reference's contract."""
     return os.environ.get("GRAPHPOPE_OUTPUT", "cpu")
 
 
@@ -298,8 +301,11 @@ def get_geodesic_distance_vector(data, num_workers):
     """utils.py:116-126: float32 ``[N, K]`` of ``1/(hops(node -> anchor)+1)``, 0 when unreachable.
 
     Reads ``data.anchor_nodes``.  Always float32 (the reference yields int64 in the degenerate case
-    where every entry is 0, SURVEY.md App. A #3).
+    where every entry is 0, SURVEY.md App. A #3).  Under ``GRAPHPOPE_OUTPUT=compact`` a
+    :class:`device.FeatureStore` with F = 0 (no cache file is read or written).
     """
+    if _output_device() == "compact":
+        return _compact_features(data, None)
     blk, path = _cached_block(data)
     if blk is not None:
         return blk.cuda() if _output_device() == "cuda" else blk
@@ -326,6 +332,20 @@ def _device_features(data, x):
     return out
 
 
+def _compact_features(data, x):
+    """``GRAPHPOPE_OUTPUT=compact``: the device-resident result as a :class:`device.FeatureStore` (x on the device,
+    the anchor block packed); the dense ``[N, F+K]`` matrix is never formed."""
+    if _shared_world() is not None:
+        raise ValueError("GRAPHPOPE_OUTPUT=compact keeps a private store per GPU; it cannot be combined with "
+                         "GRAPHPOPE_SHARED=1 in a multi-rank job")
+    if x is not None and x.dtype != torch.float32:
+        raise TypeError(f"GRAPHPOPE_OUTPUT=compact needs float32 data.x (got {x.dtype}): concat_into_features would "
+                        "type-promote the anchor block")
+    store = _dev.FeatureStore.build(_edge_index_of(data), int(data.num_nodes), data.anchor_nodes, x, SYMMETRIZE)
+    last_stats.update(store.stats)
+    return store
+
+
 def concat_into_features(embedding_matrix, data):
     """utils.py:129-135: ``torch.cat((data.x, embedding), 1)``."""
     emb = torch.as_tensor(embedding_matrix)
@@ -335,7 +355,8 @@ def concat_into_features(embedding_matrix, data):
 
 
 def attach_distance_embedding(data, dataset, num_anchor_nodes, sampling_method, distance_function, num_workers):
-    """utils.py:137-147.  Sets ``data.anchor_nodes``; returns a new CPU float32 ``[N, F + K]``.
+    """utils.py:137-147.  Sets ``data.anchor_nodes``; returns a new CPU float32 ``[N, F + K]`` (a device tensor or a
+    :class:`device.FeatureStore` under ``GRAPHPOPE_OUTPUT=cuda`` / ``compact``).
 
     Distance block and concat are one fused C-ABI call (the epilogue writes the ``[N, F+K]`` rows once).
     """
@@ -344,6 +365,10 @@ def attach_distance_embedding(data, dataset, num_anchor_nodes, sampling_method, 
                                             sampling_method=sampling_method)
     _say('deriving shortest paths to anchor nodes...')
     x = data.x
+    if _output_device() == "compact":
+        out = _compact_features(data, x)
+        _say('feature matrix is blessed by the POPE!')
+        return out
     if x.dtype != torch.float32 or _cache_dir() is not None:
         # torch.cat type-promotes; keep that behaviour by taking the generic route (also the cached one:
         # the cache holds the [N, K] block, not the concatenation)
@@ -400,7 +425,7 @@ def attach_node2vec(data, dataset, num_anchor_nodes, sampling_method, distance_f
             anchor_emb, _, _ = _dev.kmeans(table, num_anchor_nodes)
         _say('K means cluster anchor nodes derived!')
     block = _dev.cdist_minmax(table, anchor_emb, mode, apply_minmax=True)
-    out = concat_into_features(block if _output_device() == "cuda" else block.cpu(), data)
+    out = concat_into_features(block if _output_device() in ("cuda", "compact") else block.cpu(), data)
     _say('feature matrix is blessed by the POPE')
     return out
 

@@ -249,6 +249,27 @@ int gp_exchange_set_grid(gp_exchange_t *xchg, int32_t max_blocks);
 int gp_exchange_trace(gp_exchange_t *xchg, uint64_t *h_stamps8);
 int gp_exchange_free(gp_exchange_t *xchg);
 
+/* ------------------------------------------------------------------ compact feature store
+ * The anchor block of the [N, F+K] matrix in P bits per entry instead of 32, and the trainer's mini-batch lookup
+ * x[n_id] (main.py:120,177) served from it.  A store is uint64 [N][P][W], W = ceil(K/64), one contiguous record per
+ * node: plane 0 = reached mask, plane 1 + q = bit q of the hop count; column j is word j >> 6, bit j & 63 of a plane.
+ * P = 1 + bit_length(max hop) (1..17).  Padding bits past K and hop bits of unreached lanes are zero.  The value of
+ * column j is 1/(hops+1) in IEEE fp32 if reached, else 0 (bit-equal to gp_msbfs_features).  The caller owns the
+ * store buffer.                                                                                                  */
+/* syncs.  P and W of the store for the last gp_msbfs_run on bfs (bytes = N * P * W * 8). */
+int gp_fstore_layout(gp_msbfs_t *bfs, int32_t *num_planes, int64_t *words_per_plane, gp_stream_t stream);
+/* syncs.  Packs the last result into d_store [N][num_planes][W]; GP_ERR_INVALID if num_planes is too small (or
+ * above 17).  The store does not refer to bfs afterwards (the handle may be rerun or freed).                    */
+int gp_fstore_pack(gp_msbfs_t *bfs, uint64_t *d_store, int32_t num_planes, gp_stream_t stream);
+/* async.  Mini-batch rows of concat_into_features(x, features) (utils.py:129-135) as main.py:120,177 index them:
+ *   d_out[i*ld_out + c]              = d_x[rows[i]*ld_x + c]     c in [0, F)   (skipped if d_x == NULL)
+ *   d_out[i*ld_out + col_offset + j] = value of column j of node rows[i], j in [0, K)
+ * A negative id wraps once (rows[i] + N, as torch indexing does).  An id outside [-N, N) gets an all-zero output
+ * row and increments *d_bad_rows (optional device int32 counter); nothing is loaded for it.                      */
+int gp_fstore_gather(const uint64_t *d_store, int64_t num_nodes, int64_t num_anchors, int32_t num_planes,
+                     const int64_t *d_rows, int64_t num_rows, const float *d_x, int64_t num_features, int64_t ld_x,
+                     float *d_out, int64_t ld_out, int64_t col_offset, int32_t *d_bad_rows, gp_stream_t stream);
+
 /* async.  Stand-alone epilogue from a uint16 hop matrix (utils.py:73,76,125). */
 int gp_normalize_into(const uint16_t *d_dist, int64_t num_nodes, int64_t num_anchors, int64_t ld_dist,
                       float *d_out, int64_t ld_out, int64_t col_offset, gp_stream_t stream);
