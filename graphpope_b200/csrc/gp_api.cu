@@ -74,14 +74,7 @@ const GpEnv &gp_env()
         };
         GpEnv e;
         e.use_graph = geti("GP_USE_GRAPH", 1);
-        e.xcopy_overlap = geti("GP_XCOPY_OVERLAP", 0);
-        e.xcopy_stages = geti("GP_XCOPY_STAGES", 4);
-        e.xcopy_grid = geti("GP_XCOPY_GRID", 0);
-        e.bfs_cfg = geti("GP_BFS_CFG", -1);
-        e.bfs_no_map = getenv("GP_BFS_NO_MAP") != nullptr;
-        e.bfs_mapg = getenv("GP_BFS_MAPG") != nullptr;
         e.bfs_trace = getenv("GP_BFS_TRACE") != nullptr;
-        e.bfs_push = geti("GP_BFS_PUSH", 0);
         e.xchg_grid = geti("GP_XCHG_GRID", 0);
         e.xchg_debug = geti("GP_XCHG_DEBUG", 0);
         e.stage_events = geti("GP_STAGE_EVENTS", 0);
@@ -398,79 +391,28 @@ namespace {
 
 thread_local bool g_capturing = false;  // a capture belongs to the thread that runs it
 
-struct SideCopy {
-    cudaStream_t stream = nullptr;
-    cudaEvent_t fork = nullptr, join = nullptr;
-};
-
-SideCopy &side_copy_state()
-{
-    static thread_local SideCopy sc;
-    return sc;
-}
-
 int run_pipeline_eager(gp_csr *csr, gp_msbfs *bfs, const int64_t *d_ei, int64_t e, const int64_t *d_anchors,
                        int64_t k, const float *d_x, int64_t f, int64_t ldx, float *d_out, int64_t ldo,
                        int64_t coff, cudaStream_t s, gp_exchange *xchg = nullptr, int parity = 0)
 {
-    // concat_into_features' copy of x (utils.py:133-134) depends on neither the csr build nor the traversal, which
-    // are latency-bound and leave HBM idle, so it could run beside them on a side stream (a parallel branch of the
-    // captured graph).  Measured on B200 it never pays: whatever moves the rows — the copy engine (round 1), copy
-    // kernels of three shapes (round 1), or the bulk-copy-engine pipeline of gp_xcopy.cu (round 2: 4.9 TB/s alone,
-    // one thread and 64 KB of shared memory per SM, resident next to the cooperative MS-BFS grid) — the latency-bound
-    // neighbours slow down by about the time the copy takes (csr build 94 -> 153-170 us, msbfs_kernel 86 -> 117-241 us
-    // while rows stream through the L2, even throttled to 3.6 TB/s; profiles/r02_notes.md), so the copy stays fused
-    // in the epilogue kernel (GP_XCOPY_OVERLAP=0, default).  1 = one strided cudaMemcpy2DAsync on the copy engine,
-    // 2 = the bulk-copy kernel on the side branch.
-    const int overlap = gp_env().xcopy_overlap;
-    const bool have_copy = d_out != nullptr && d_x != nullptr && f > 0 && csr->num_nodes > 0 && xchg == nullptr;
-    const bool tma_copy = have_copy && overlap == 2 && gp_xcopy_tma_ok(d_x, f, ldx, d_out, ldo);
-    const bool side_copy = have_copy && (overlap == 1 || tma_copy);
-    SideCopy &sc = side_copy_state();
-    if (side_copy) {
-        if (sc.stream == nullptr) {
-            GP_CUDA_CHECK(cudaStreamCreateWithFlags(&sc.stream, cudaStreamNonBlocking));
-            GP_CUDA_CHECK(cudaEventCreateWithFlags(&sc.fork, cudaEventDisableTiming));
-            GP_CUDA_CHECK(cudaEventCreateWithFlags(&sc.join, cudaEventDisableTiming));
-        }
-        GP_CUDA_CHECK(cudaEventRecord(sc.fork, s));
-        GP_CUDA_CHECK(cudaStreamWaitEvent(sc.stream, sc.fork, 0));
-        int crc = GP_OK;
-        if (tma_copy) {
-            crc = gp_launch_xcopy_tma(d_x, csr->num_nodes, f, ldx, d_out, ldo, sc.stream);
-        } else if (cudaMemcpy2DAsync(d_out, (size_t)ldo * sizeof(float), d_x, (size_t)ldx * sizeof(float),
-                                     (size_t)f * sizeof(float), (size_t)csr->num_nodes, cudaMemcpyDeviceToDevice,
-                                     sc.stream) != cudaSuccess) {
-            gp_set_error("cudaMemcpy2DAsync of x failed");
-            crc = GP_ERR_CUDA;
-        }
-        GP_CUDA_CHECK(cudaEventRecord(sc.join, sc.stream));  // always re-join: a capture must not end forked
-        if (crc != GP_OK) {
-            cudaStreamWaitEvent(s, sc.join, 0);
-            return crc;
-        }
-    }
+    // concat_into_features' copy of x (utils.py:133-134) stays fused in the epilogue kernel.  It depends on neither the
+    // csr build nor the traversal, but run beside them on a side stream it slows them by about its own duration,
+    // whatever moves the rows (profiles/r02_notes.md).
     // stage clocks of the step (gp_pipeline_stage_ms): inside a capture these become event-record nodes
     const unsigned ev_flags = gp_is_capturing() ? cudaEventRecordExternal : cudaEventRecordDefault;
     const bool stage_events = gp_stage_events_on(bfs);
     if (stage_events) GP_CUDA_CHECK(cudaEventRecordWithFlags(bfs->ev_pipe0, s, ev_flags));
-    int rc;
     {
         GpRange r("graphpope:csr_build");
-        rc = gp_csr_build(csr, d_ei, e, s);
+        GP_TRY(gp_csr_build(csr, d_ei, e, s));
     }
-    if (rc == GP_OK) {
+    {
         GpRange r("graphpope:msbfs");
-        bfs->push_edges = d_ei;  // the caller's edge buffer is alive for this call: hop 1 may scan it (push direction)
-        bfs->push_num_edges = e;
-        rc = gp_msbfs_run(bfs, d_anchors, k, s);
-        bfs->push_edges = nullptr;
+        GP_TRY(gp_msbfs_run(bfs, d_anchors, k, s));
     }
-    if (side_copy) GP_CUDA_CHECK(cudaStreamWaitEvent(s, sc.join, 0));  // always re-join: a capture must not end forked
-    GP_TRY(rc);
     GpRange r(xchg != nullptr ? "graphpope:exchange_decode" : "graphpope:epilogue");
     if (xchg != nullptr) GP_TRY(gp_exchange_launch(xchg, parity, d_x, f, ldx, d_out, ldo, coff, s));
-    else if (d_out != nullptr) GP_TRY(gp_msbfs_features(bfs, side_copy ? nullptr : d_x, f, ldx, d_out, ldo, coff, s));
+    else if (d_out != nullptr) GP_TRY(gp_msbfs_features(bfs, d_x, f, ldx, d_out, ldo, coff, s));
     else GP_TRY(gp_msbfs_pack(bfs, (int32_t)coff, nullptr, nullptr, nullptr, nullptr, nullptr, s));  // coff = slot
     if (stage_events) GP_CUDA_CHECK(cudaEventRecordWithFlags(bfs->ev_pipe1, s, ev_flags));
     bfs->pipe_timed = stage_events;

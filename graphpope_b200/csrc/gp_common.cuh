@@ -50,14 +50,7 @@ int gp_sm_count();  // cached multiProcessorCount of the current device
 // around as plain data afterwards: no getenv on any call path, no function-local caches.
 struct GpEnv {
     int use_graph;       // GP_USE_GRAPH (default 1): replay the fused pipeline from a CUDA graph
-    int xcopy_overlap;   // GP_XCOPY_OVERLAP (default 0): where the x copy of concat runs (gp_api.cu)
-    int xcopy_stages;    // GP_XCOPY_STAGES (default 4)
-    int xcopy_grid;      // GP_XCOPY_GRID (default 0 = one block per SM)
-    int bfs_cfg;         // GP_BFS_CFG (default GP_BFS_DEFAULT_CFG): MS-BFS launch shape
-    int bfs_no_map;      // GP_BFS_NO_MAP: per-hop bitmaps off
-    int bfs_mapg;        // GP_BFS_MAPG: per-hop bitmaps read from global memory
     int bfs_trace;       // GP_BFS_TRACE: per-level clocks
-    int bfs_push;        // GP_BFS_PUSH (default 0): hop 1 in push direction, as a scan of the raw edge list (measured slower)
     int xchg_grid;       // GP_XCHG_GRID: cap on the exchange kernel's grid (tests: several ranks on one GPU)
     int xchg_debug;      // GP_XCHG_DEBUG
     int stage_events;    // GP_STAGE_EVENTS (default 0): event NODES around csr / bfs / epilogue inside captured pipelines

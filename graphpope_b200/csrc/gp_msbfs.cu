@@ -71,9 +71,6 @@ struct BfsParams {
     int *status;
     u64 *counters;
     u64 *trace;                     // optional per-warp phase clocks (diagnostics), else nullptr
-    const long long *push_ei;       // raw edge_index [2][push_e] for the hop-1 push (fused pipeline only), else nullptr
-    long long push_e;
-    int push_sym;                   // the CSR was built with GP_CSR_SYMMETRIZE: every edge also counts reversed
 };
 
 template <int VW>
@@ -216,11 +213,16 @@ __device__ __forceinline__ bool finalize_row(const LevelCtx<VW> &c, size_t off, 
     return incomplete;
 }
 
-// Warp-iterations cached per CTA: enough for GP_BFS_CACHE_ITERS * 24 tiles per SM whatever the launch shape.
-__host__ __device__ constexpr int bfs_cache_iters(int nt, int minb)
-{
-    return (GP_BFS_CACHE_ITERS * 24 + (nt / 32) * minb - 1) / ((nt / 32) * minb);
-}
+// Launch shape: 384 threads x 2 CTAs per SM (80 registers) ties 768x1 as the fastest; fewer warps run 5% slower, more
+// warps spill (profiles/r01k_notes.md).
+constexpr int BFS_THREADS = 384;
+constexpr int BFS_CTAS_PER_SM = 2;
+constexpr int BFS_WARPS = BFS_THREADS / 32;
+// Tiles of a CTA whose work items live in shared memory: GP_BFS_CACHE_ITERS per warp.
+constexpr int BFS_CACHED_TILES = GP_BFS_CACHE_ITERS * BFS_WARPS;
+constexpr size_t BFS_CACHE_BYTES =
+    (size_t)BFS_CACHED_TILES * 32 * (2 * sizeof(int4) + GP_BFS_DONE_BATCHES) + (size_t)BFS_CACHED_TILES * GP_BFS_DONE_BATCHES;
+static_assert((BFS_CACHED_TILES * GP_BFS_DONE_BATCHES) % 16 == 0, "the staged bitmaps that follow are read as uint4");
 
 // Descriptor and column indices of the 32 slots of tile `t0 / 32` (one degree class per tile).
 //   lead = {row or -1, count | chunks << 8 | first << 30, hub index, log2 G}, cols = <= 4 columns or -1.
@@ -246,88 +248,14 @@ __device__ __forceinline__ void load_tile(const BfsParams &p, const int *s_ent_b
     cols = make_int4(c[0], c[1], c[2], c[3]);
 }
 
-// ---- hop 1 in PUSH direction.  The frontier is the K anchors: pulling makes every row look its neighbours up in the
-// anchor bitmap (7-8 K cycles for the 2 K rows that find one).  Instead the raw edge list the CSR was built from is
-// scanned once, coalesced: an edge u -> a whose head is an anchor pushes the anchor's lanes into row u with L2
-// reductions (duplicate edges are idempotent).  Needs the bitmaps and the edge list, i.e. the fused pipeline; one
-// lane-word batch (K <= 256 per GPU).  Kept out of line so its registers do not weigh on the pull loop.  Returns the
-// number of rows pushed to (an upper bound: a row reached over two edges counts twice; it only sizes the next
-// level's filter).
-template <int WB>
-__device__ __noinline__ int push_hop1(const long long *push_ei, long long push_e, int push_sym, int n, const u64 *seeds,
-                                      u64 *counters, long long gtid, long long gthreads, const u32 *map0, u32 *map_w,
-                                      u64 *nxt, u64 *seen, u32 *s_live32, int *s_any)
-{
-    constexpr int VW = WB;
-    const int lane = threadIdx.x & 31;
-    int nzrows = 0;
-    u64 pushes = 0;
-    auto is_anchor = [&](int v) { return ((map0[v >> 5] >> (v & 31)) & 1u) != 0; };
-    // One edge whose head v is an anchor: the tail index and the anchor's lane words are requested together, the row
-    // is updated with reductions nobody waits for.
-    auto push_edge = [&](const long long *tail, int v) {
-        u64 lanes[VW], mine[VW];
-        vload<VW>(seeds + (size_t)v * WB, lanes);
-        const long long uu = __ldg(tail);
-        if ((unsigned long long)uu >= (unsigned long long)n) return;
-        const int u = (int)uu;
-        const size_t ou = (size_t)u * WB;
-#pragma unroll
-        for (int i = 0; i < VW; ++i) mine[i] = 0;
-        if (is_anchor(u)) vload<VW>(seeds + ou, mine);  // u is an anchor itself: its hop-0 lanes
-        bool any = false;
-#pragma unroll
-        for (int i = 0; i < VW; ++i) {
-            const u64 nw = lanes[i] & ~mine[i];
-            if (nw) {
-                any = true;
-                red_or_u64(nxt + ou + i, nw);
-                red_or_u64(seen + ou + i, nw);
-                atomicOr(&s_live32[i * 2], (u32)nw);
-                atomicOr(&s_live32[i * 2 + 1], (u32)(nw >> 32));
-            }
-        }
-        if (any) {
-            *s_any = 1;
-            red_or_u32(map_w + (u >> 5), 1u << (u & 31));
-            ++nzrows;
-            pushes += VW;
-        }
-    };
-    const long long *src = push_ei, *dst = push_ei + push_e;
-    constexpr int PE = 8;  // edges per thread and trip: one round trip for the whole Flickr-size scan
-    for (long long i0 = gtid; i0 < push_e; i0 += PE * gthreads) {
-        int d[PE];  // node ids fit 32 bits; -1 = out of range (latched by the csr build) or past the end
-#pragma unroll
-        for (int q = 0; q < PE; ++q) {
-            const long long i = i0 + q * gthreads;
-            const long long v = i < push_e ? __ldg(dst + i) : -1;
-            d[q] = (unsigned long long)v < (unsigned long long)n ? (int)v : -1;
-        }
-#pragma unroll
-        for (int q = 0; q < PE; ++q)
-            if (d[q] >= 0 && is_anchor(d[q])) push_edge(src + i0 + q * gthreads, d[q]);
-        if (push_sym) {  // the reversed copy of every edge (GP_CSR_SYMMETRIZE)
-#pragma unroll 1
-            for (int q = 0; q < PE; ++q) {
-                const long long i = i0 + q * gthreads;
-                const long long v = i < push_e ? __ldg(src + i) : -1;
-                if ((unsigned long long)v < (unsigned long long)n && is_anchor((int)v)) push_edge(dst + i, (int)v);
-            }
-        }
-    }
-    for (int m = 16; m; m >>= 1) pushes += shfl_xor_u64(pushes, m);
-    if (lane == 0 && pushes) atomicAdd(counters + 1, pushes);
-    return nzrows;
-}
-
 // WB lane words per node row = one thread loads a whole row (8, 16 or 32 bytes).
-template <int WB, int NT, int MINB, bool MAPG, bool PUSH>
-__global__ void __launch_bounds__(NT, MINB) msbfs_kernel(BfsParams p)
+template <int WB, bool MAPG>
+__global__ void __launch_bounds__(BFS_THREADS, BFS_CTAS_PER_SM) msbfs_kernel(BfsParams p)
 {
     constexpr int VW = WB;
-    constexpr int WARPS = NT / 32;
-    constexpr int JT = bfs_cache_iters(NT, MINB) * WARPS;  // tiles of this CTA whose work items live in shared memory
+    constexpr int NT = BFS_THREADS;
+    constexpr int WARPS = BFS_WARPS;
+    constexpr int JT = BFS_CACHED_TILES;
     static_assert(GP_SLOT_EDGES == 4, "slot layout is int4");
     // Work cache: a CTA visits the same tiles every level, so the descriptors and column indices of
     // its first JT tiles are loaded ONCE into shared memory; a level then costs a single dependent
@@ -482,20 +410,7 @@ __global__ void __launch_bounds__(NT, MINB) msbfs_kernel(BfsParams p)
         GP_TRACE(0);
 
         int nzrows = 0;
-        // ---- hop 1 in PUSH direction.  The frontier is the K anchors: pulling makes every row look its neighbours up
-        // in the anchor bitmap (7 K cycles for 2 K rows that find one).  Instead the raw edge list the CSR was built
-        // from is scanned once, coalesced: an edge u -> a whose head is an anchor pushes the anchor's lanes into row
-        // u with L2 reductions (duplicate edges are idempotent).  Needs the bitmaps and the edge list (fused pipeline).
-        // hop 1 in push direction (GP_BFS_PUSH=1, fused pipeline, one lane-word batch): see push_hop1
-        const bool push_level = PUSH && level == 1 && map_level;
-        if constexpr (PUSH) {
-            if (push_level) {
-                nzrows += push_hop1<WB>(p.push_ei, p.push_e, p.push_sym, n, p.seeds, p.counters, gtid, gthreads,
-                                        MAPG ? p.nzmap : s_map, map_w, c.nxt, c.seen, s_live32, &s_any);
-                s_notdone = 1;  // no row has been tested for completeness at this hop
-            }
-        }
-        for (int b = 0; b < (push_level ? 0 : p.batches); ++b) {
+        for (int b = 0; b < p.batches; ++b) {
             u64 lv[VW], live_acc[VW];
 #pragma unroll
             for (int i = 0; i < VW; ++i) {
@@ -661,54 +576,44 @@ __global__ void __launch_bounds__(NT, MINB) msbfs_kernel(BfsParams p)
         asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
         p.counters[3] = t;
         p.status[GP_BFS_ST_MAX_LEVEL] = max_level;
-        const int pushed = (PUSH && use_map) ? 1 : 0;
         p.status[GP_BFS_ST_LEVELS] = level;
-        p.status[GP_BFS_ST_PULL] = level - pushed;
-        p.status[GP_BFS_ST_PUSH] = pushed;
     }
 }
 
-template <int WB, int NT, int MINB>
-constexpr size_t bfs_cache_bytes()
+// Frontier bitmaps are staged in shared memory when they fit next to the work cache without costing a resident CTA;
+// bitmaps too large for shared memory are read from global memory by the MAPG variant.
+template <int WB>
+int launch_bfs(gp_msbfs *h, const BfsParams &p, cudaStream_t stream)
 {
-    constexpr int tiles = bfs_cache_iters(NT, MINB) * (NT / 32);
-    static_assert((tiles * GP_BFS_DONE_BATCHES) % 16 == 0, "the staged bitmaps that follow are read as uint4");
-    return (size_t)tiles * 32 * (2 * sizeof(int4) + GP_BFS_DONE_BATCHES) + (size_t)tiles * GP_BFS_DONE_BATCHES;
-}
-
-template <int WB, int NT, int MINB, bool MAPG, bool PUSH>
-int launch_bfs_variant(gp_msbfs *h, const BfsParams &p, cudaStream_t stream, int cfg_id)
-{
-    // Frontier bitmaps are staged in shared memory when they fit without costing a resident CTA.
     const int want_map = (int)((size_t)p.map_stride * sizeof(u32));
-    const int key = ((cfg_id * 8 + WB) * 4 + 1 + (MAPG ? 2 : 0)) * 2 + (PUSH ? 1 : 0);
+    const bool mapg = BFS_CACHE_BYTES + (size_t)p.map_stride * sizeof(u32) > 200 * 1024 / (size_t)BFS_CTAS_PER_SM;
+    void (*const kernel)(BfsParams) = mapg ? msbfs_kernel<WB, true> : msbfs_kernel<WB, false>;
+    const int key = WB * 2 + (mapg ? 1 : 0);
     if (h->grid_blocks == 0 || h->grid_cfg != key || h->map_want_bytes != want_map) {
         int occ = 0, occ_map = 0;
         cudaFuncAttributes fa;
-        GP_CUDA_CHECK(cudaFuncGetAttributes(&fa, msbfs_kernel<WB, NT, MINB, MAPG, PUSH>));
+        GP_CUDA_CHECK(cudaFuncGetAttributes(&fa, kernel));
         int smem_optin = 0, dev = 0;
         GP_CUDA_CHECK(cudaGetDevice(&dev));
         GP_CUDA_CHECK(cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
         const int dyn_room = smem_optin - (int)fa.sharedSizeBytes;
-        const int cache_bytes = (int)bfs_cache_bytes<WB, NT, MINB>();
+        const int cache_bytes = (int)BFS_CACHE_BYTES;
         int dyn_max = cache_bytes + GP_BFS_MAP_SMEM_MAX;
         if (dyn_max > dyn_room) dyn_max = dyn_room;
         GP_REQUIRE(dyn_max >= cache_bytes, GP_ERR_CUDA, "msbfs work cache does not fit in shared memory");
-        GP_CUDA_CHECK(cudaFuncSetAttribute(msbfs_kernel<WB, NT, MINB, MAPG, PUSH>, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_max));
-        GP_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, msbfs_kernel<WB, NT, MINB, MAPG, PUSH>, NT,
-                                                                    bfs_cache_bytes<WB, NT, MINB>()));
+        GP_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn_max));
+        GP_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, BFS_THREADS, BFS_CACHE_BYTES));
         GP_REQUIRE(occ >= 1, GP_ERR_CUDA, "msbfs kernel does not fit on an SM");
-        if (occ > MINB) occ = MINB;
+        if (occ > BFS_CTAS_PER_SM) occ = BFS_CTAS_PER_SM;
         h->map_smem_bytes = 0;
-        if (!MAPG && cache_bytes + want_map <= dyn_max && !gp_env().bfs_no_map) {
-            GP_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_map, msbfs_kernel<WB, NT, MINB, MAPG, PUSH>, NT,
-                                                                        bfs_cache_bytes<WB, NT, MINB>() + want_map));
+        if (!mapg && cache_bytes + want_map <= dyn_max) {
+            GP_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_map, kernel, BFS_THREADS,
+                                                                        BFS_CACHE_BYTES + want_map));
             if (occ_map >= occ) h->map_smem_bytes = want_map;
         }
         h->grid_blocks = occ * gp_sm_count();
         h->grid_cfg = key;
         h->map_want_bytes = want_map;
-        h->block_threads = NT;
     }
     BfsParams pp = p;
     pp.map_smem_words = h->map_smem_bytes > 0 ? p.map_stride : 0;
@@ -718,49 +623,11 @@ int launch_bfs_variant(gp_msbfs *h, const BfsParams &p, cudaStream_t stream, int
     const unsigned ev_flags = gp_is_capturing() ? cudaEventRecordExternal : cudaEventRecordDefault;
     h->kernel_timed = gp_stage_events_on(h);
     if (h->kernel_timed) GP_CUDA_CHECK(cudaEventRecordWithFlags(h->ev_start, stream, ev_flags));
-    GP_CUDA_CHECK(cudaLaunchCooperativeKernel((const void *)msbfs_kernel<WB, NT, MINB, MAPG, PUSH>, dim3(h->grid_blocks),
-                                              dim3(NT), args, bfs_cache_bytes<WB, NT, MINB>() + h->map_smem_bytes, stream));
+    GP_CUDA_CHECK(cudaLaunchCooperativeKernel((const void *)kernel, dim3(h->grid_blocks), dim3(BFS_THREADS), args,
+                                              BFS_CACHE_BYTES + h->map_smem_bytes, stream));
     if (h->kernel_timed) GP_CUDA_CHECK(cudaEventRecordWithFlags(h->ev_stop, stream, ev_flags));
     return GP_OK;
 }
-
-// The shared-memory variant when the bitmaps fit next to the work cache, else (default shape only) the
-// variant that reads them from global memory.
-template <int WB, int NT, int MINB>
-int launch_bfs_cfg(gp_msbfs *h, const BfsParams &p, cudaStream_t stream, int cfg_id)
-{
-    const size_t want_map = (size_t)p.map_stride * sizeof(u32);
-    const bool fits = bfs_cache_bytes<WB, NT, MINB>() + want_map <= 200 * 1024 / (size_t)MINB;
-    const bool force_global = gp_env().bfs_mapg != 0;  // experiment: never stage the maps
-    // the push variant exists for the default launch shape only (it is an experiment that lost: profiles/r02_notes.md)
-    const bool push = p.push_ei != nullptr && p.batches <= GP_BFS_PUSH_BATCHES && cfg_id == GP_BFS_DEFAULT_CFG &&
-                      !gp_env().bfs_no_map;
-    if ((!fits || force_global) && cfg_id == GP_BFS_DEFAULT_CFG && !gp_env().bfs_no_map)
-        return push ? launch_bfs_variant<WB, NT, MINB, true, NT == 384 && MINB == 2>(h, p, stream, cfg_id)
-                    : launch_bfs_variant<WB, NT, MINB, true, false>(h, p, stream, cfg_id);
-    return push ? launch_bfs_variant<WB, NT, MINB, false, NT == 384 && MINB == 2>(h, p, stream, cfg_id)
-                : launch_bfs_variant<WB, NT, MINB, false, false>(h, p, stream, cfg_id);
-}
-
-// Launch shapes (threads per CTA, CTAs per SM) trade resident warps against registers per thread,
-// i.e. against how many neighbour gathers one thread keeps in flight.  GP_BFS_CFG picks one.
-template <int WB>
-int launch_bfs(gp_msbfs *h, const BfsParams &p, cudaStream_t stream)
-{
-    int cfg = gp_env().bfs_cfg;
-    if (cfg < 0 || cfg > 7) cfg = GP_BFS_DEFAULT_CFG;
-    switch (cfg) {
-        case 0: return launch_bfs_cfg<WB, 768, 1>(h, p, stream, 0);   // 85 regs, 24 warps/SM, one tile queue per SM
-        case 1: return launch_bfs_cfg<WB, 384, 2>(h, p, stream, 1);   // 85 regs, 24 warps/SM
-        case 2: return launch_bfs_cfg<WB, 512, 1>(h, p, stream, 2);   // 128 regs, 16 warps/SM
-        case 3: return launch_bfs_cfg<WB, 1024, 1>(h, p, stream, 3);  // 64 regs, 32 warps/SM
-        case 4: return launch_bfs_cfg<WB, 512, 2>(h, p, stream, 4);   // 64 regs, 32 warps/SM, two queues
-        case 5: return launch_bfs_cfg<WB, 320, 2>(h, p, stream, 5);   // 102 regs, 20 warps/SM
-        case 6: return launch_bfs_cfg<WB, 256, 2>(h, p, stream, 6);   // 128 regs, 16 warps/SM
-        default: return launch_bfs_cfg<WB, 640, 1>(h, p, stream, 7);  // 102 regs, 20 warps/SM, one queue
-    }
-}
-
 }  // namespace
 
 static void bfs_config(int64_t k, int *wb, int *batches)
@@ -910,7 +777,7 @@ extern "C" int gp_msbfs_run(gp_msbfs_t *h, const int64_t *d_anchors, int64_t num
     p.nzmap = h->nzmap;
     p.nzwords = (int)h->nzwords;
     p.map_stride = map_stride;
-    p.map_smem_words = 0;  // decided per launch configuration (launch_bfs_cfg)
+    p.map_smem_words = 0;  // decided by launch_bfs
     p.col = h->csr->col;
     p.meta = h->csr->meta;
     p.anchors = (const long long *)d_anchors;
@@ -924,9 +791,6 @@ extern "C" int gp_msbfs_run(gp_msbfs_t *h, const int64_t *d_anchors, int64_t num
     p.status = h->status;
     p.counters = h->counters;
     p.trace = h->trace;
-    p.push_ei = (h->push_hop1 < 0 ? gp_env().bfs_push : h->push_hop1) ? (const long long *)h->push_edges : nullptr;
-    p.push_e = h->push_num_edges;
-    p.push_sym = (h->csr->flags & GP_CSR_SYMMETRIZE) ? 1 : 0;
     GP_TRY(wb == 1 ? launch_bfs<1>(h, p, stream) : wb == 2 ? launch_bfs<2>(h, p, stream)
                                                              : launch_bfs<4>(h, p, stream));
     h->ran = true;
@@ -963,12 +827,11 @@ extern "C" int gp_msbfs_kernel_device_ns(gp_msbfs_t *h, uint64_t *ns, gp_stream_
     return GP_OK;
 }
 
+// Hop 1 always pulls; the entry point stays for programs built against ABI version 1.
 extern "C" int gp_msbfs_set_push(gp_msbfs_t *h, int32_t enable)
 {
     GP_REQUIRE(h != nullptr, GP_ERR_INVALID, "gp_msbfs_set_push: handle is NULL");
-    h->push_hop1 = enable ? 1 : 0;
-    gp_pipe_cache_free(h->pipe_cache);  // captured pipelines hold the other kernel variant
-    h->pipe_cache = nullptr;
+    GP_REQUIRE(enable == 0, GP_ERR_UNSUPPORTED, "gp_msbfs_set_push: hop 1 always pulls; push direction is not supported");
     return GP_OK;
 }
 
@@ -989,9 +852,9 @@ extern "C" int gp_msbfs_stats(gp_msbfs_t *h, gp_msbfs_stats_t *stats, gp_stream_
     stats->lane_words = (int64_t)h->wb * h->batches;
     stats->max_level = st[GP_BFS_ST_MAX_LEVEL];
     stats->levels_run = st[GP_BFS_ST_LEVELS];
-    stats->pull_levels = st[GP_BFS_ST_PULL];
-    stats->push_levels = st[GP_BFS_ST_PUSH];
-    stats->edges_examined = (int64_t)cnt[0] + (int64_t)cnt[1];
+    stats->pull_levels = st[GP_BFS_ST_LEVELS];  // every level pulls
+    stats->push_levels = 0;
+    stats->edges_examined = (int64_t)cnt[0];
     stats->grid_blocks = h->grid_blocks;
     GP_REQUIRE(!(csr_err & GP_DEV_ERR_EDGE_RANGE), GP_ERR_INDEX_RANGE,
                "edge_index holds an entry outside [0, %lld)", (long long)h->num_nodes);
@@ -1010,7 +873,7 @@ extern "C" int gp_msbfs_trace(gp_msbfs_t *h, uint64_t *h_out, int64_t cap_words,
     gp_msbfs_stats(h, &st, nullptr);
     GP_CUDA_CHECK(cudaDeviceSynchronize());
     *levels = st.levels_run < 32 ? st.levels_run : 32;
-    *warps = h->grid_blocks * (h->block_threads / 32);
+    *warps = h->grid_blocks * BFS_WARPS;
     const int64_t words = (int64_t)32 * (*warps) * 4;  // all 32 rows: row 31 holds the prologue stamps of shallow runs
     GP_REQUIRE(words <= cap_words && words <= GP_BFS_TRACE_WORDS, GP_ERR_INVALID, "gp_msbfs_trace: buffer too small");
     GP_CUDA_CHECK(cudaMemcpy(h_out, h->trace, sizeof(u64) * (size_t)words, cudaMemcpyDeviceToHost));

@@ -3,13 +3,11 @@
 
 #include "gp_internal.h"
 
-constexpr int GP_BFS_DEFAULT_CFG = 1;       // see launch_bfs in gp_msbfs.cu
 constexpr int GP_BFS_MAX_LANE_WORDS = 256;  // B * WB cap (K <= 16384 per GPU)
 constexpr int GP_BFS_PLANES = 16;           // deep-hop distance bit planes (uint16 range)
 constexpr int GP_BFS_LEVEL_ARRAYS = 15;     // hops 1..15 are recorded as write-once frontier arrays
 constexpr int GP_BFS_CACHE_ITERS = 4;      // warp-iterations whose work items are cached in shared memory
 constexpr int GP_BFS_MAP_SMEM_MAX = 64 * 1024;  // largest set of frontier bitmaps staged in shared memory
-constexpr int GP_BFS_PUSH_BATCHES = 1;     // hop 1 runs in push direction for up to this many lane-word batches
 constexpr int GP_BFS_DONE_BATCHES = 8;     // batches that keep per-row "done" flags for cached items
 constexpr int GP_MAX_RANKS = 8;             // GPUs of one NVSwitch node
 constexpr int GP_BFS_RESULT_ARRAYS = 1 + GP_BFS_LEVEL_ARRAYS + GP_BFS_PLANES;  // 32
@@ -19,8 +17,6 @@ enum : int {
     GP_BFS_ST_MAX_LEVEL = 0,
     GP_BFS_ST_ERROR = 1,
     GP_BFS_ST_LEVELS = 2,
-    GP_BFS_ST_PULL = 3,
-    GP_BFS_ST_PUSH = 4,
     GP_BFS_ST_WORDS = 8
 };
 
@@ -58,19 +54,13 @@ struct gp_msbfs {
     int map_want_bytes = -1; // map size the cached launch configuration was computed for
     int64_t hub_capacity = 0;
     bool hub_zeroed = false;
-    // raw edge_index the CSR was just built from, valid for the next gp_msbfs_run only (set by the fused pipeline,
-    // which holds the caller's buffer): lets hop 1 run in push direction
-    int push_hop1 = -1;  // hop 1 in push direction: -1 = GP_BFS_PUSH (default off), 0 / 1 = gp_msbfs_set_push
-    const int64_t *push_edges = nullptr;
-    int64_t push_num_edges = 0;
     u64 *packed = nullptr;   // [2 slots][GP_PACKED_ARRAYS][cap words] exchange buffers (allocated on first pack)
     int *deep_flag = nullptr;  // device int: 1 if the last packed run had hops > 15 (packed format invalid)
     int *status = nullptr;      // [GP_BFS_ST_WORDS]
-    u64 *counters = nullptr;    // [4] gathers issued, pushes issued, ...
+    u64 *counters = nullptr;    // [4] gathers issued, unused, %globaltimer at kernel entry and after the last level
     u64 *trace = nullptr;       // [32 levels][warps][4] phase clocks, only with GP_BFS_TRACE=1
     int grid_blocks = 0;
-    int grid_cfg = -1;
-    int block_threads = 512;
+    int grid_cfg = -1;          // kernel variant (WB, MAPG) the cached grid size was computed for
     cudaEvent_t ev_start = nullptr, ev_stop = nullptr;  // bracket the persistent kernel alone
     cudaEvent_t ev_pipe0 = nullptr, ev_pipe1 = nullptr;  // first / last node of the last gp_geodesic_run pipeline
     bool pipe_timed = false;   // the last fused run recorded ev_pipe0 / ev_pipe1

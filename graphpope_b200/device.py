@@ -189,10 +189,6 @@ class MsBfs:
                                           _ptr(out), ld_out, f, _stream()))
         return out
 
-    def set_push(self, enable: bool):
-        """Hop 1 of the fused pipeline in push direction (an edge scan from the anchors) instead of pull."""
-        check(self._lib.gp_msbfs_set_push(self._h, int(bool(enable))))
-
     def stats(self) -> dict:
         st = MsbfsStats()
         check(self._lib.gp_msbfs_stats(self._h, byref(st), _stream()))

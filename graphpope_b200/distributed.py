@@ -488,7 +488,6 @@ class PullAssembly:
             self._opened.append(ptr.value)
         self.step = 0
         self.trace_events = []
-        self._side = None
         self.flag = torch.zeros(1, dtype=torch.int32, device="cuda")
 
     def close(self):
@@ -518,19 +517,6 @@ class PullAssembly:
             self._shard_key, self._shard = key, anchors[lo:hi].contiguous()
         edge_index = edge_index.contiguous()
         eng.csr._edges, eng.bfs._anchors, eng.bfs.num_anchors = edge_index, self._shard, hi - lo
-        # concat_into_features' copy of x (utils.py:133-134) does not depend on the traversal; opt-in
-        # (GP_XCOPY_OVERLAP=1): one strided device-to-device transfer on a side stream while this rank builds,
-        # traverses and packs.  Off by default: on one GPU the overlapped forms measured slower than the fused copy.
-        side = None
-        if x is not None and f > 0 and n > 0 and os.environ.get("GP_XCOPY_OVERLAP", "0") != "0":
-            if self._side is None:
-                self._side = torch.cuda.Stream()
-            side = self._side
-            side.wait_stream(torch.cuda.current_stream())
-            check(self.lib.gp_concat_x(_ptr(x), n, f, x.stride(0) if n > 1 else f, _ptr(out),
-                                       out.stride(0) if n > 1 else f + k, c_void_p(side.cuda_stream)))
-            x.record_stream(side)
-            out.record_stream(side)
         trace = os.environ.get("GP_PEER_TRACE") is not None  # diagnostics: device time of the three phases
         if trace:
             ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
@@ -553,9 +539,6 @@ class PullAssembly:
         for r in range(self.world):
             base = packed.value - slot * self.slot_stride_words * 8 if r == self.rank else self.base[r]
             ptrs[r] = base + slot * self.slot_stride_words * 8
-        if side is not None:
-            torch.cuda.current_stream().wait_stream(side)
-            x = None  # already in place
         check(self.lib.gp_decode_peers(ptrs, self.world, n, hi - lo, batches.value, wb.value, stride.value, _ptr(x), f,
                                        x.stride(0) if x is not None and n > 1 else f, _ptr(out),
                                        out.stride(0) if n > 1 else f + k, f, _stream()))

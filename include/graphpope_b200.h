@@ -80,9 +80,9 @@ typedef struct gp_msbfs_stats {
     int64_t lane_words;        /* uint64 lane words per node (64 anchors each)   */
     int32_t max_level;         /* largest finite hop distance                    */
     int32_t levels_run;        /* level sweeps executed                          */
-    int32_t pull_levels;
-    int32_t push_levels;
-    int64_t edges_examined;    /* neighbour lane-word gathers + pushes issued    */
+    int32_t pull_levels;       /* = levels_run: every level pulls                */
+    int32_t push_levels;       /* 0                                              */
+    int64_t edges_examined;    /* neighbour lane-word gathers issued             */
     int64_t grid_blocks;       /* persistent grid size                           */
 } gp_msbfs_stats_t;
 
@@ -133,9 +133,8 @@ int gp_msbfs_hops_u16(gp_msbfs_t *bfs, uint16_t *d_dist, int64_t ld, int64_t col
  * IEEE fp32 division (bit-equal to the reference's float64 -> float32 rounding). */
 int gp_msbfs_features(gp_msbfs_t *bfs, const float *d_x, int64_t num_features, int64_t ld_x,
                       float *d_out, int64_t ld_out, int64_t col_offset, gp_stream_t stream);
-/* Direction of hop 1 inside gp_geodesic_run (the fused call holds the raw edge list): 1 = PUSH, an edge scan from the
- * anchors with L2 reductions; 0 = pull like every other hop (default: on the named graphs the pull sweep, which finds
- * its column indices in shared memory, is as fast; profiles/r02_notes.md).  Results are identical either way.     */
+/* Hop 1 pulls like every other hop (a push form measured slower; profiles/r02_notes.md).  Kept for programs built
+ * against ABI version 1: enable == 0 returns GP_OK, any other value GP_ERR_UNSUPPORTED.                          */
 int gp_msbfs_set_push(gp_msbfs_t *bfs, int32_t enable);
 /* syncs.  Reports latched GP_ERR_INDEX_RANGE / GP_ERR_LEVEL_OVERFLOW. */
 int gp_msbfs_stats(gp_msbfs_t *bfs, gp_msbfs_stats_t *stats, gp_stream_t stream);
@@ -164,12 +163,11 @@ int gp_msbfs_set_stage_events(gp_msbfs_t *bfs, int32_t enable);
 int gp_msbfs_kernel_device_ns(gp_msbfs_t *bfs, uint64_t *ns, gp_stream_t stream);
 int gp_pipeline_stage_ms(gp_msbfs_t *bfs, float *ms3);
 
-/* async.  The x half of concat_into_features (utils.py:133-134) alone: d_out[:, 0:F] = d_x as ONE strided
- * device-to-device transfer, for callers that already hold x in place or want the copy on their own stream;
- * follow with gp_msbfs_features / gp_decode_peers called with d_x == NULL.  gp_geodesic_run keeps the copy
- * inside the epilogue kernel by default: running it beside the csr build and the MS-BFS measured slower on
- * B200 (copy engine 0.323 ms, copy kernels 0.265-0.301 ms, against 0.246 ms per step; GP_XCOPY_OVERLAP=1
- * selects the copy-engine variant).                                                                    */
+/* async.  The x half of concat_into_features (utils.py:133-134) alone: d_out[:, 0:F] = d_x (a bulk-copy kernel for
+ * 16-byte aligned rows, else one strided device-to-device transfer), for callers that want the copy on their own
+ * stream; follow with gp_msbfs_features / gp_decode_peers called with d_x == NULL.  gp_geodesic_run keeps the copy
+ * inside its epilogue kernel: running it beside the csr build and the MS-BFS measured slower on B200 (copy engine
+ * 0.323 ms, copy kernels 0.265-0.301 ms, against 0.246 ms per step).                                           */
 int gp_concat_x(const float *d_x, int64_t num_nodes, int64_t num_features, int64_t ld_x, float *d_out,
                 int64_t ld_out, gp_stream_t stream);
 

@@ -94,7 +94,8 @@ def test_csr_row_sort_paths(dev, n):
     s_, d_ = g.dedup_edges(ei, n, False)
     assert info["num_edges"] == s_.size
     assert info["max_out_degree"] == np.bincount(s_, minlength=n).max()
-    # and the traversal over that CSR (hub chunks, every slot class) stays bit-exact
+    # and the traversal over that CSR (hub chunks, every slot class) stays bit-exact; at n = 1_000_000 the per-hop
+    # bitmaps (125 KB) do not fit in shared memory next to the work cache, so this runs the global-memory map variant
     anchors = rng.integers(0, n, 64)
     hops, _, _ = _gpu_hops_and_features(dev, ei, n, anchors)
     assert np.array_equal(hops, _oracle_hops(ei, n, anchors))
@@ -558,10 +559,12 @@ def test_two_hundred_runs_are_identical(dev, flickr):
 
 @pytest.mark.parametrize("symmetrize", [False, True])
 @pytest.mark.parametrize("k", [1, 64, 100, 256])
-def test_hop1_push_direction_matches_pull_and_oracle(dev, k, symmetrize):
-    """gp_msbfs_set_push: hop 1 of the fused pipeline as a push (edge scan from the anchors, L2 reductions) on an
-    asymmetric multigraph with self loops and repeated edges, duplicate anchors and anchors adjacent to anchors; with
-    and without GP_CSR_SYMMETRIZE.  Bit-equal to the pull result and to the oracle; the stats report one push level."""
+def test_hop1_pull_matches_oracle(dev, k, symmetrize):
+    """Hop 1 of the fused pipeline pulls like every other hop, on an asymmetric multigraph with self loops and repeated
+    edges, duplicate anchors and anchors adjacent to anchors; with and without GP_CSR_SYMMETRIZE.  Bit-equal to the
+    oracle on the eager, captured and replayed runs; the stats report no push level.  gp_msbfs_set_push keeps its ABI
+    version 1 symbol: 0 is accepted, 1 is GP_ERR_UNSUPPORTED."""
+    from graphpope_b200 import _lib
     n = 5000
     ei = np.concatenate([synth.chung_lu_symmetric(n, 30000, 2.2, seed=13), synth.random_digraph(n, 4000, seed=14)], axis=1)
     rng = np.random.default_rng(k)
@@ -572,14 +575,16 @@ def test_hop1_push_direction_matches_pull_and_oracle(dev, k, symmetrize):
     want = _oracle_hops(ei, n, anchors, symmetrize)
     ei_d, a_d = torch.as_tensor(ei).cuda(), torch.as_tensor(anchors).cuda()
     eng = dev.GeodesicEngine(n, ei.shape[1], k, symmetrize)
-    for push in (True, False):
-        eng.bfs.set_push(push)
-        for _ in range(3):  # eager, captured, replayed
-            eng.run(ei_d, a_d)
+    lib = _lib.load()
+    assert lib.gp_msbfs_set_push(eng.bfs._h, 1) == _lib.GP_ERR_UNSUPPORTED
+    assert b"always pulls" in lib.gp_last_error()
+    assert lib.gp_msbfs_set_push(eng.bfs._h, 0) == _lib.GP_OK
+    for run in ("eager", "captured", "replayed"):
+        eng.run(ei_d, a_d)
         hops = eng.bfs.hops_u16().cpu().numpy()
         st = eng.bfs.stats()
-        assert np.array_equal(hops, want), push
-        assert st["push_levels"] == (1 if push else 0) and st["pull_levels"] + st["push_levels"] == st["levels_run"]
+        assert np.array_equal(hops, want), run
+        assert st["push_levels"] == 0 and st["pull_levels"] + st["push_levels"] == st["levels_run"], run
 
 
 @pytest.mark.parametrize("k", [50, 3, 64])

@@ -12,7 +12,7 @@ ei = synth.make_graph(shape); anchors = synth.stochastic_anchors(n, K, 42)
 ei_d = torch.as_tensor(ei).cuda(); a_d = torch.as_tensor(anchors).cuda()
 eng = dev.GeodesicEngine(n, ei.shape[1], K); eng.bfs.set_stage_events(True)
 out = torch.empty(n, K, device="cuda")
-fused = os.environ.get("GP_TRACE_FUSED", "1") != "0"  # the fused pipeline hands the edge list to the kernel (hop-1 push)
+fused = os.environ.get("GP_TRACE_FUSED", "1") != "0"  # trace the fused pipeline (csr build + MS-BFS), else the MS-BFS alone
 run = (lambda: eng.run(ei_d, a_d, None, out)) if fused else (lambda: eng.bfs.run(a_d))
 eng.csr.build(ei_d)
 for _ in range(3): run()

@@ -1,9 +1,9 @@
-"""Bulk-copy-engine x copy (gp_xcopy.cu): rate alone, and the pipeline step with / without it beside csr + bfs."""
+"""Bulk-copy-engine x copy (gp_xcopy.cu, gp_concat_x) against torch's strided copy_ at the Flickr shape."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from ctypes import c_void_p
-from graphpope_b200 import device as dev, synth, _lib
+from graphpope_b200 import synth, _lib
 lib = _lib.load()
 sh = synth.SHAPES["flickr-shape"]; n, f, k = sh.num_nodes, sh.num_features, 256
 x = torch.randn(n, f, device="cuda"); out = torch.empty(n, f + k, device="cuda")
@@ -19,53 +19,6 @@ st = lambda: c_void_p(torch.cuda.current_stream().cuda_stream)
 cp = lambda: _lib.check(lib.gp_concat_x(c_void_p(x.data_ptr()), n, f, f, c_void_p(out.data_ptr()), f + k, st()))
 for _ in range(3): cp()
 med, mn = timed(cp)
-print(f"GP_XCOPY_STAGES={os.environ.get('GP_XCOPY_STAGES','4')}: x copy alone {med*1e3:.1f} us median ({mn*1e3:.1f} min) = {8*n*f/med/1e6:.0f} GB/s", flush=True)
+print(f"gp_concat_x {med*1e3:.1f} us median ({mn*1e3:.1f} min) = {8*n*f/med/1e6:.0f} GB/s", flush=True)
 med, mn = timed(lambda: out[:, :f].copy_(x))
 print(f"torch strided copy_ {med*1e3:.1f} us = {8*n*f/med/1e6:.0f} GB/s", flush=True)
-ei = synth.make_graph(sh); anchors = synth.stochastic_anchors(n, k, 42)
-ei_d = torch.as_tensor(ei).cuda(); a_d = torch.as_tensor(anchors).cuda()
-eng = dev.GeodesicEngine(n, ei.shape[1], k); eng.bfs.set_stage_events(True)
-for _ in range(4): eng.run(ei_d, a_d, x, out)
-med, mn = timed(lambda: eng.run(ei_d, a_d, x, out))
-print(f"GP_XCOPY_OVERLAP={os.environ.get('GP_XCOPY_OVERLAP','2')}: step {med*1e3:.1f} us median ({mn*1e3:.1f} min), msbfs kernel {eng.bfs.kernel_ms()*1e3:.1f} us", flush=True)
-for _ in range(4): eng.run(ei_d, a_d, None, out)
-med, mn = timed(lambda: eng.run(ei_d, a_d, None, out))
-print(f"step without x: {med*1e3:.1f} us median ({mn*1e3:.1f} min), msbfs kernel {eng.bfs.kernel_ms()*1e3:.1f} us", flush=True)
-# ---- phases under overlap, launched by hand: copy on a side stream, csr -> bfs -> features on the main one
-side = torch.cuda.Stream()
-def phases(with_copy):
-    res = []
-    for i in range(12):
-        flush.fill_(float(i)); s = flush[:1024].sum(); torch.cuda.synchronize()
-        ev = [torch.cuda.Event(enable_timing=True) for _ in range(6)]
-        ev[0].record()
-        if with_copy:
-            side.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(side):
-                ev[4].record(); cp(); ev[5].record()
-        eng.csr.build(ei_d); ev[1].record(); eng.bfs.run(a_d); ev[2].record()
-        if with_copy: torch.cuda.current_stream().wait_stream(side)
-        eng.bfs.features(None, out); ev[3].record(); torch.cuda.synchronize()
-        row = [ev[0].elapsed_time(ev[1]), ev[1].elapsed_time(ev[2]), ev[2].elapsed_time(ev[3]), ev[0].elapsed_time(ev[3])]
-        if with_copy: row += [ev[0].elapsed_time(ev[4]), ev[4].elapsed_time(ev[5])]
-        res.append(row)
-    return np.median(np.array(res), axis=0) * 1e3
-print("eager phases us, no copy   [csr, bfs, decode, total]:", np.round(phases(False), 1), flush=True)
-print("eager phases us, with copy [csr, bfs, decode, total, copy start, copy dur]:", np.round(phases(True), 1), "bfs kernel", round(eng.bfs.kernel_ms()*1e3, 1), flush=True)
-def phases_bfs_only():
-    res = []
-    for i in range(12):
-        flush.fill_(float(i)); s = flush[:1024].sum(); torch.cuda.synchronize()
-        ev = [torch.cuda.Event(enable_timing=True) for _ in range(6)]
-        ev[0].record()
-        eng.csr.build(ei_d); ev[1].record()
-        side.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(side):
-            ev[4].record(); cp(); ev[5].record()
-        eng.bfs.run(a_d); ev[2].record()
-        torch.cuda.current_stream().wait_stream(side)
-        eng.bfs.features(None, out); ev[3].record(); torch.cuda.synchronize()
-        res.append([ev[0].elapsed_time(ev[1]), ev[1].elapsed_time(ev[2]), ev[2].elapsed_time(ev[3]), ev[0].elapsed_time(ev[3]),
-                    ev[0].elapsed_time(ev[4]), ev[4].elapsed_time(ev[5]), eng.bfs.kernel_ms()])
-    return np.median(np.array(res), axis=0) * 1e3
-print("copy beside the BFS only   [csr, bfs, decode, total, copy start, copy dur, bfs kernel]:", np.round(phases_bfs_only(), 1), flush=True)
