@@ -105,6 +105,7 @@ SIGNATURES = {
     "gp_exchange_free": (c_int, [c_void_p]),
     "gp_fstore_layout": (c_int, [c_void_p, POINTER(c_int32), POINTER(c_int64), c_void_p]),
     "gp_fstore_pack": (c_int, [c_void_p, c_void_p, c_int32, c_void_p]),
+    "gp_fstore_merge": (c_int, [c_void_p, c_int32, c_int64, c_int64, c_int64, c_int32, c_int64, c_void_p, c_void_p]),
     "gp_fstore_gather": (c_int, [c_void_p, c_int64, c_int64, c_int32, c_void_p, c_int64, c_void_p, c_int64, c_int64,
                                  c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
     "gp_normalize_into": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64, c_int64, c_void_p]),

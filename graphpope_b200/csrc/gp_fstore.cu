@@ -50,6 +50,48 @@ __global__ void __launch_bounds__(256) fstore_pack_kernel(const u64 *__restrict_
     }
 }
 
+// One thread per destination word (record row r = node * P + plane, word w): the shards of `per` columns each that
+// overlap columns [64w, 64w + 64) are ORed in, each through at most two of its own words funnel-shifted into place
+// and masked to its column range.  Shard and store rows share the [N][P] row order, so the row index carries over.
+// When per % 64 == 0 every shift is zero and exactly one shard covers a word: the merge is a word permutation.
+__global__ void __launch_bounds__(256) fstore_merge_kernel(const u64 *__restrict__ shards, long long per,
+                                                           long long shard_words, long long rows, long long words,
+                                                           long long k, u64 *__restrict__ store)
+{
+    const long long step = (long long)gridDim.x * blockDim.x;
+    const long long i0 = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long step_r = step / words, step_w = step - step_r * words;
+    long long r = i0 / words, w = i0 - r * words;
+    const size_t shard_stride = (size_t)rows * shard_words;
+    while (r < rows) {
+        const long long c0 = w << 6;
+        const long long c1 = c0 + 64 < k ? c0 + 64 : k;
+        u64 v = 0;
+        for (long long s = c0 / per, s_last = (c1 - 1) / per; s <= s_last; ++s) {
+            const long long base = s * per;
+            const long long cnt = k - base < per ? k - base : per;  // columns shard s holds
+            const long long off = c0 - base;  // shard column of destination bit 0; in (-64, 0) if s starts mid-word
+            const long long a = off >> 6;     // floor: -1 when off < 0
+            const int sh = (int)(off & 63);
+            const int t0 = off < 0 ? (int)-off : 0;
+            const int t1 = cnt - off < 64 ? (int)(cnt - off) : 64;
+            const long long last = (cnt - 1) >> 6;  // last shard word holding columns of s
+            const u64 *src = shards + (size_t)s * shard_stride + (size_t)r * shard_words;
+            u64 x = a >= 0 ? __ldg(src + a) >> sh : 0ull;
+            if (sh != 0 && a + 1 <= last) x |= __ldg(src + a + 1) << (64 - sh);
+            const u64 mask = (t1 == 64 ? ~0ull : (1ull << t1) - 1) & (~0ull << t0);
+            v |= x & mask;
+        }
+        store[(size_t)r * words + w] = v;
+        w += step_w;
+        r += step_r;
+        if (w >= words) {
+            w -= words;
+            ++r;
+        }
+    }
+}
+
 struct FsGather {
     const u64 *store;
     long long n, k, words;  // nodes, anchors, uint64 words per plane
@@ -235,6 +277,31 @@ extern "C" int gp_fstore_pack(gp_msbfs_t *h, uint64_t *d_store, int32_t num_plan
               (long long)h->num_nodes, h->wb, (int)words, levels, deep, (int)num_planes, (u64 *)d_store);
     GP_CUDA_CHECK(cudaGetLastError());
     GP_CUDA_CHECK(cudaStreamSynchronize(stream));  // the store must not depend on bfs once this returns
+    return GP_OK;
+}
+
+extern "C" int gp_fstore_merge(const uint64_t *d_shards, int32_t num_shards, int64_t cols_per_shard,
+                               int64_t words_per_shard, int64_t num_nodes, int32_t num_planes, int64_t num_anchors,
+                               uint64_t *d_store, gp_stream_t stream_)
+{
+    GP_REQUIRE(num_shards >= 1 && cols_per_shard >= 0 && num_nodes >= 0 && num_anchors >= 0, GP_ERR_INVALID,
+               "gp_fstore_merge: bad shape arguments");
+    GP_REQUIRE(num_planes >= 1 && num_planes <= FS_MAX_PLANES, GP_ERR_INVALID,
+               "gp_fstore_merge: num_planes %d outside [1, %d]", (int)num_planes, FS_MAX_PLANES);
+    GP_REQUIRE(words_per_shard >= (cols_per_shard + 63) / 64, GP_ERR_INVALID,
+               "gp_fstore_merge: %lld words per shard plane cannot hold %lld columns", (long long)words_per_shard,
+               (long long)cols_per_shard);
+    GP_REQUIRE((int64_t)num_shards * cols_per_shard >= num_anchors, GP_ERR_INVALID,
+               "gp_fstore_merge: %d shards of %lld columns cannot hold %lld anchors", (int)num_shards,
+               (long long)cols_per_shard, (long long)num_anchors);
+    const int64_t words = (num_anchors + 63) / 64;
+    if (num_nodes == 0 || words == 0) return GP_OK;
+    GP_REQUIRE(d_shards != nullptr && d_store != nullptr, GP_ERR_INVALID, "gp_fstore_merge: NULL argument");
+    const long long rows = num_nodes * num_planes;
+    GP_LAUNCH(fstore_merge_kernel, fs_grid(rows * words, 256), 256, 0, (cudaStream_t)stream_, (const u64 *)d_shards,
+              (long long)cols_per_shard, (long long)words_per_shard, rows, (long long)words, (long long)num_anchors,
+              (u64 *)d_store);
+    GP_CUDA_CHECK(cudaGetLastError());
     return GP_OK;
 }
 

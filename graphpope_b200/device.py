@@ -290,25 +290,59 @@ class FeatureStore:
     documented in include/graphpope_b200.h, gp_fstore_*).  Rows are produced on demand by a fused gather kernel, so
     ``store[n_id]`` stands in for ``data.x[n_id]`` of the trainer (main.py:120,177) without the dense matrix.
 
-    ``FeatureStore(bfs, x)`` packs the last run of an :class:`MsBfs` (the store does not refer to it afterwards).
+    ``FeatureStore(bfs, x)`` packs the last run of an :class:`MsBfs` (the store does not refer to it afterwards);
+    ``num_planes`` packs with more planes than the run needs (the extra hop bits are zero), so that stores of
+    different anchor shards share one layout.  :meth:`from_shards` merges such shard stores into one.
     """
 
-    def __init__(self, bfs: MsBfs, x: torch.Tensor | None = None):
+    def __init__(self, bfs: MsBfs, x: torch.Tensor | None = None, num_planes: int | None = None):
         self._lib = _lib.require_cuda()
-        n, k = bfs.csr.num_nodes, bfs.num_anchors
+        n = bfs.csr.num_nodes
+        x = self._device_x(x, n)
+        stats = bfs.stats()  # syncs; surfaces index errors of the run
+        planes, words = c_int32(), c_int64()
+        check(self._lib.gp_fstore_layout(bfs._h, byref(planes), byref(words), _stream()))
+        p = planes.value if num_planes is None else int(num_planes)  # too few planes: GP_ERR_INVALID from the pack
+        raw = torch.empty((n, p, words.value), dtype=torch.uint64, device="cuda")
+        check(self._lib.gp_fstore_pack(bfs._h, _ptr(raw), p, _stream()))
+        self._adopt(raw, bfs.num_anchors, x, stats)
+
+    @staticmethod
+    def _device_x(x, n):
         if x is not None:
             if x.dtype != torch.float32 or x.dim() != 2 or x.size(0) != n:
                 raise TypeError("x must be a float32 tensor of shape [N, F]")
             x = x.to(device="cuda").contiguous()
-        self.stats = bfs.stats()  # syncs; surfaces index errors of the run
-        planes, words = c_int32(), c_int64()
-        check(self._lib.gp_fstore_layout(bfs._h, byref(planes), byref(words), _stream()))
-        self._raw = torch.empty((n, planes.value, words.value), dtype=torch.uint64, device="cuda")
-        check(self._lib.gp_fstore_pack(bfs._h, _ptr(self._raw), planes.value, _stream()))
-        self._x = x
-        self.num_nodes, self.num_anchors = n, k
+        return x
+
+    def _adopt(self, raw, k, x, stats):
+        self._raw, self._x, self.stats = raw, x, stats
+        self.num_nodes, self.num_anchors = raw.size(0), int(k)
         self.num_features = 0 if x is None else x.size(1)
         self._bad = torch.zeros(1, dtype=torch.int32, device="cuda")
+
+    @classmethod
+    def from_shards(cls, shards: torch.Tensor, num_anchors: int, x: torch.Tensor | None = None,
+                    stats: dict | None = None) -> "FeatureStore":
+        """One store from the stores of S contiguous anchor shards, stacked as a cuda uint64 (or int64) tensor
+        ``[S, N, P, Ws]``: shard s holds anchors ``distributed.shard_bounds(K, S, s)``, i.e. columns
+        ``[s * ceil(K/S), min((s + 1) * ceil(K/S), K))``, packed with the common P and zero-padded to Ws >=
+        ceil(ceil(K/S) / 64) words.  ``raw`` is byte-identical to that of one run over all K anchors packed with P
+        planes (``FeatureStore.build`` when P is what the deepest shard needs).  Runs on the current stream."""
+        lib = _lib.require_cuda()
+        if not shards.is_cuda or shards.dim() != 4 or shards.dtype not in (torch.uint64, torch.int64):
+            raise TypeError("shards must be a cuda uint64 tensor [S, N, P, Ws]")
+        shards = shards.contiguous()
+        s, n, p, ws = shards.shape
+        k = int(num_anchors)
+        per = -(-k // s) if s else 0
+        x = cls._device_x(x, n)
+        raw = torch.empty((n, p, -(-k // 64)), dtype=torch.uint64, device="cuda")
+        check(lib.gp_fstore_merge(_ptr(shards), s, per, ws, n, p, k, _ptr(raw), _stream()))
+        store = cls.__new__(cls)
+        store._lib = lib
+        store._adopt(raw, k, x, {} if stats is None else dict(stats))
+        return store
 
     @classmethod
     def build(cls, edge_index, num_nodes: int, anchors, x: torch.Tensor | None = None,

@@ -64,6 +64,118 @@ def gather_planes(local_planes: torch.Tensor, group=None) -> torch.Tensor:
     return out.view((world,) + tuple(local_planes.shape))
 
 
+def anchor_checksum(anchors) -> int:
+    """A 62-bit digest of the anchor list (count and values, in order), non-negative in an int64."""
+    import hashlib
+
+    import numpy as np
+
+    a = np.ascontiguousarray(np.asarray(torch.as_tensor(anchors).cpu(), dtype=np.int64).reshape(-1))
+    h = hashlib.blake2b(np.int64([a.size]).tobytes() + a.tobytes(), digest_size=8).digest()
+    return int.from_bytes(h, "little") >> 2
+
+
+def check_anchors_agree(anchors, group=None, device="cpu"):
+    """Raises ``ValueError`` on every rank unless every rank passed the same anchor list: all-reduce MIN and MAX of
+    :func:`anchor_checksum`.  A sharded build from different lists would silently mix columns of different runs."""
+    c = anchor_checksum(anchors)
+    lo = torch.tensor([c], dtype=torch.int64, device=device)
+    hi = lo.clone()
+    dist.all_reduce(lo, op=dist.ReduceOp.MIN, group=group)
+    dist.all_reduce(hi, op=dist.ReduceOp.MAX, group=group)
+    if int(lo.item()) != int(hi.item()):
+        raise ValueError("the ranks passed different anchor lists to a collective anchor-sharded build (same seed "
+                         "and sampler on every rank are needed)")
+
+
+def agree_store_layout(local_num_planes: int, local_max_level: int, failed: bool = False, group=None,
+                       device="cpu") -> tuple[int, int, bool]:
+    """(P, max_level, some rank failed): the max over ranks of each, in one all-reduce.  The largest finite hop over
+    all shards is the one-GPU ``max_level``, so the agreed P is the one a single run over all anchors packs with."""
+    t = torch.tensor([int(local_num_planes), int(local_max_level), int(bool(failed))], dtype=torch.int64,
+                     device=device)
+    dist.all_reduce(t, op=dist.ReduceOp.MAX, group=group)
+    p, level, bad = t.tolist()
+    return int(p), int(level), bool(bad)
+
+
+def shard_words(num_anchors: int, world_size: int) -> int:
+    """Ws: uint64 words per plane of every rank's shard store, enough for the ``ceil(K/G)`` anchors of a full
+    shard, so that all ranks' blocks have one shape for the all-gather."""
+    per = -(-int(num_anchors) // int(world_size))
+    return -(-per // 64)
+
+
+def pad_shard_store(raw: torch.Tensor | None, num_nodes: int, num_planes: int, words: int,
+                    device="cpu") -> torch.Tensor:
+    """A shard store ``[N, P_local, W_local]`` (``None``: a rank without anchors) as an int64 ``[N, P, Ws]`` block,
+    zero in the planes and words it lacks; the store itself (viewed as int64) when it already has that shape."""
+    shape = (int(num_nodes), int(num_planes), int(words))
+    if raw is not None and tuple(raw.shape) == shape:
+        return raw.view(torch.int64)
+    block = torch.zeros(shape, dtype=torch.int64, device=raw.device if raw is not None else device)
+    if raw is not None:
+        block[:, :raw.size(1), :raw.size(2)].copy_(raw.view(torch.int64))
+    return block
+
+
+def sharded_feature_store(edge_index, num_nodes: int, anchors, x: torch.Tensor | None = None,
+                          symmetrize: bool = False, group=None):
+    """Collective: every rank calls it with the same arguments and gets the same :class:`device.FeatureStore` of all
+    K anchors, whose ``raw`` is byte-identical to ``FeatureStore.build(edge_index, num_nodes, anchors, x)`` on one
+    GPU.  Rank r runs the csr build and the MS-BFS for its anchors ``shard_bounds(K, G, r)`` only (a BFS workspace of
+    ``ceil(K/G)`` lanes), packs them with the P agreed over the ranks into a zero-padded ``[N, P, Ws]`` block, frees
+    the BFS workspace, all-gathers the G blocks and merges them into the one-GPU record layout (gp_fstore_merge).
+    Peak device memory is about twice the store plus x.  ``store.stats`` holds this rank's MS-BFS counters with
+    ``max_level`` the max over the ranks.  Needs a process group that all-gathers cuda tensors (NCCL)."""
+    import numpy as np
+
+    from ._lib import MsbfsStats
+    from .device import DeviceCsr, FeatureStore, MsBfs
+
+    backend = str(dist.get_backend(group))
+    if "nccl" not in backend:
+        raise RuntimeError(f"sharded_feature_store all-gathers cuda tensors and needs an NCCL process group, "
+                           f"not {backend!r}")
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    a = np.ascontiguousarray(np.asarray(torch.as_tensor(anchors).cpu(), dtype=np.int64).reshape(-1))
+    n, k = int(num_nodes), a.size
+    check_anchors_agree(a, group, device="cuda")
+    lo, hi = shard_bounds(k, world, rank)
+    ws = shard_words(k, world)
+    csr = bfs = None
+    stats = MsbfsStats().as_dict()  # a rank without anchors: all counters zero
+    error = None
+    try:
+        ei = torch.as_tensor(edge_index).to(device="cuda", dtype=torch.int64)
+        if ei.dim() != 2 or ei.size(0) != 2:
+            raise ValueError("edge_index must have shape [2, E]")
+        if hi > lo:
+            csr = DeviceCsr(n, ei.size(1), symmetrize).build(ei)
+            bfs = MsBfs(csr, hi - lo).run(torch.from_numpy(a[lo:hi]).cuda())
+            stats = bfs.stats()  # syncs; surfaces index errors of the run
+    except Exception as e:  # reported to the other ranks below instead of leaving them in a collective
+        error = e
+    local_planes = 1 + int(stats["max_level"]).bit_length()
+    try:
+        p, max_level, failed = agree_store_layout(local_planes, stats["max_level"], error is not None, group, "cuda")
+        if error is not None:
+            raise error
+        if failed:
+            raise RuntimeError("sharded_feature_store failed on another rank")
+        shard = FeatureStore(bfs, num_planes=p).raw if bfs is not None else None
+    finally:
+        for h in (bfs, csr):
+            if h is not None:
+                h.close()
+    block = pad_shard_store(shard, n, p, ws, device="cuda")
+    del shard
+    gathered = gather_planes(block, group)  # [G, N, P, Ws] int64
+    del block
+    stats = dict(stats, max_level=max_level)
+    return FeatureStore.from_shards(gathered, k, x, stats)
+
+
 def _wrap_device_words(ptr: int, nwords: int) -> torch.Tensor:
     """Zero-copy int64 view of library-owned device memory (the bit planes of the last run)."""
     class _Holder:

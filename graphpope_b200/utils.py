@@ -334,14 +334,19 @@ def _device_features(data, x):
 
 def _compact_features(data, x):
     """``GRAPHPOPE_OUTPUT=compact``: the device-resident result as a :class:`device.FeatureStore` (x on the device,
-    the anchor block packed); the dense ``[N, F+K]`` matrix is never formed."""
-    if _shared_world() is not None:
-        raise ValueError("GRAPHPOPE_OUTPUT=compact keeps a private store per GPU; it cannot be combined with "
-                         "GRAPHPOPE_SHARED=1 in a multi-rank job")
+    the anchor block packed); the dense ``[N, F+K]`` matrix is never formed.  With ``GRAPHPOPE_SHARED=1`` in a
+    multi-rank job the ranks split the anchors: each runs the MS-BFS for its ``K/G`` of them, and every rank ends up
+    holding the same whole store (``distributed.sharded_feature_store``)."""
     if x is not None and x.dtype != torch.float32:
         raise TypeError(f"GRAPHPOPE_OUTPUT=compact needs float32 data.x (got {x.dtype}): concat_into_features would "
                         "type-promote the anchor block")
-    store = _dev.FeatureStore.build(_edge_index_of(data), int(data.num_nodes), data.anchor_nodes, x, SYMMETRIZE)
+    if _shared_world() is not None:
+        from . import distributed as _gpd
+
+        store = _gpd.sharded_feature_store(_edge_index_of(data), int(data.num_nodes), data.anchor_nodes, x,
+                                           SYMMETRIZE)
+    else:
+        store = _dev.FeatureStore.build(_edge_index_of(data), int(data.num_nodes), data.anchor_nodes, x, SYMMETRIZE)
     last_stats.update(store.stats)
     return store
 

@@ -259,6 +259,15 @@ int gp_fstore_layout(gp_msbfs_t *bfs, int32_t *num_planes, int64_t *words_per_pl
 /* syncs.  Packs the last result into d_store [N][num_planes][W]; GP_ERR_INVALID if num_planes is too small (or
  * above 17).  The store does not refer to bfs afterwards (the handle may be rerun or freed).                    */
 int gp_fstore_pack(gp_msbfs_t *bfs, uint64_t *d_store, int32_t num_planes, gp_stream_t stream);
+/* async.  Merges anchor-shard stores into one store: d_shards is uint64 [S][N][P][Ws], shard s holding columns
+ * [s*cols_per_shard, min((s+1)*cols_per_shard, K)) in the store format above with Ws >= ceil(cols_per_shard/64)
+ * words per plane (tail shards may be short or empty; their words past their own columns are ignored).  Writes
+ * d_store [N][P][ceil(K/64)], byte-identical to the store of one run over all K anchors packed with P planes.
+ * GP_ERR_INVALID, before any CUDA call, if P is outside [1, 17], Ws < ceil(cols_per_shard/64),
+ * S*cols_per_shard < K, or a pointer is NULL while N*K > 0.                                                     */
+int gp_fstore_merge(const uint64_t *d_shards, int32_t num_shards, int64_t cols_per_shard, int64_t words_per_shard,
+                    int64_t num_nodes, int32_t num_planes, int64_t num_anchors, uint64_t *d_store,
+                    gp_stream_t stream);
 /* async.  Mini-batch rows of concat_into_features(x, features) (utils.py:129-135) as main.py:120,177 index them:
  *   d_out[i*ld_out + c]              = d_x[rows[i]*ld_x + c]     c in [0, F)   (skipped if d_x == NULL)
  *   d_out[i*ld_out + col_offset + j] = value of column j of node rows[i], j in [0, K)
