@@ -429,14 +429,22 @@ extern "C" int gp_decode_gathered(const uint64_t *d_gathered, int64_t rank_strid
                                   int64_t ld_out, int64_t col_offset, gp_stream_t stream_)
 {
     GP_REQUIRE(d_gathered != nullptr && d_out != nullptr, GP_ERR_INVALID, "gp_decode_gathered: NULL argument");
-    GP_REQUIRE(num_ranks >= 1 && num_nodes >= 0 && anchors_per_rank >= 0 && num_planes >= 1 &&
-                   num_planes <= GP_BFS_RESULT_ARRAYS && batches >= 1 &&
+    GP_REQUIRE(num_ranks >= 1 && num_nodes >= 0 && anchors_per_rank >= 0 && batches >= 1 &&
                    (words_per_batch == 1 || words_per_batch == 2 || words_per_batch == 4),
                GP_ERR_INVALID, "gp_decode_gathered: bad shape arguments");
+    // what gp_msbfs_planes reports: 1 + max_level <= 16 planes, or all 32 once a hop exceeds 15 (the decoder then
+    // reads the 16 deep-hop planes whole, so 17..31 would read past the shard)
+    GP_REQUIRE((num_planes >= 1 && num_planes <= 1 + GP_BFS_LEVEL_ARRAYS) || num_planes == GP_BFS_RESULT_ARRAYS,
+               GP_ERR_INVALID, "gp_decode_gathered: num_planes %d is not 1..%d or %d", num_planes,
+               1 + GP_BFS_LEVEL_ARRAYS, GP_BFS_RESULT_ARRAYS);
     GP_REQUIRE(anchors_per_rank <= (int64_t)batches * words_per_batch * 64, GP_ERR_INVALID,
                "gp_decode_gathered: anchors_per_rank exceeds the lane capacity of a shard");
-    GP_REQUIRE(ld_out >= col_offset + anchors_per_rank * num_ranks, GP_ERR_INVALID,
-               "gp_decode_gathered: ld_out too small");
+    GP_REQUIRE(plane_stride_words >= (int64_t)batches * words_per_batch * num_nodes &&
+                   (num_ranks == 1 || rank_stride_words >= (int64_t)num_planes * plane_stride_words),
+               GP_ERR_INVALID, "gp_decode_gathered: plane or rank stride smaller than a plane or a shard");
+    GP_REQUIRE(num_features >= 0 && col_offset >= 0 && ld_out >= col_offset + anchors_per_rank * num_ranks &&
+                   (d_x == nullptr || (ld_x >= num_features && ld_out >= num_features)),
+               GP_ERR_INVALID, "gp_decode_gathered: inconsistent leading dimensions");
     GpDecodeParams p;
     memset(&p, 0, sizeof(p));
     p.planes0 = (const u64 *)d_gathered;

@@ -40,7 +40,7 @@ struct gp_exchange {
     size_t pk_stride = 0;          // words between packed planes (cap_words rounded up to 16-byte multiples)
     unsigned char *buf = nullptr;  // flags [2][GP_MAX_RANKS] u32 (256 B) | packed [2][5][pk_stride] u64 | pad
     unsigned char *peer[GP_MAX_RANKS] = {};  // base of every rank's buffer (own = buf)
-    u32 *local = nullptr;          // [0..1] epoch of each parity, [2..3] blocks packed, [4] deep seen, [5] timeout,
+    u32 *local = nullptr;          // [0..1] epoch of each parity, [2..3] blocks packed, [4] deep (last step), [5] timeout,
                                    // [6..7] blocks left; bytes 64..: u64 globaltimer stamps (diagnostics)
     int step = 0;
     int grid_blocks = 0;
@@ -212,13 +212,15 @@ __global__ void __launch_bounds__(XCHG_THREADS, 4) exchange_decode_kernel(XchgPa
                 }
                 any_deep |= f & 1u;
             }
-            if (timed_out) atomicExch(p.local + 5, 1u);
-            if (any_deep) atomicExch(p.local + 4, 1u);
+            if (timed_out) atomicExch(p.local + 5, 1u);  // sticky: a dead peer is fatal
+            // every block has seen the same flags: block 0 writes this step's deep bit (0 or 1), so a shallow step
+            // after a deep one reports 0
+            if (blockIdx.x == 0) p.local[4] = any_deep;
             if (gtid == 0) stamp[2] = now();
         }
         __syncthreads();
-    } else if (deep && gtid == 0) {
-        atomicExch(p.local + 4, 1u);
+    } else if (gtid == 0) {
+        p.local[4] = deep;
     }
 
     // ---- stream: one pass over the row blocks; thread 0 keeps the bulk-copy engine two blocks ahead

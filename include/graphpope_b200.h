@@ -173,14 +173,23 @@ int gp_concat_x(const float *d_x, int64_t num_nodes, int64_t num_features, int64
 
 /* Bit-sliced result planes of the last run, for the multi-GPU gather
  * (anchor-sharded ranks exchange these instead of uint16/fp32 columns):
- * plane 0 = "reached" mask, planes 1..num_planes-1 = distance bits 0.. ;
- * each plane is uint64 [batches][N][words_per_batch].  syncs (needs max_level). */
+ *   plane 0          "reached" mask;
+ *   plane l, 1..15   lanes first reached at hop l (one-hot over the planes);
+ *   plane 16 + q     bit q of the hop count of lanes first reached at hop 16 or later.
+ * num_planes = 1 + max_level (1..16) when every hop is <= 15, else 32.  Planes at or past
+ * num_planes hold stale bits of earlier runs.  Each plane is uint64
+ * [batches][N][words_per_batch].  syncs (needs max_level).                      */
 int gp_msbfs_planes(gp_msbfs_t *bfs, const uint64_t **d_planes, int64_t *plane_stride_words,
                     int32_t *num_planes, int32_t *batches, int32_t *words_per_batch, gp_stream_t stream);
 /* async.  Decode planes gathered from `num_ranks` anchor shards (each shard laid
  * out as gp_msbfs_planes reports, shard r at d_gathered + r*rank_stride_words)
  * into columns [col_offset + r*anchors_per_rank + j] of d_out, optionally
- * copying x as gp_msbfs_features does.                                          */
+ * copying x as gp_msbfs_features does.  num_planes is one value for all shards,
+ * 1..16 or 32 (the largest any shard reported); a shard that reported fewer must
+ * hold zeros in its planes up to num_planes.  GP_ERR_INVALID, before any CUDA
+ * call, for other num_planes, plane_stride_words < batches*words_per_batch*N,
+ * rank_stride_words < num_planes*plane_stride_words (more than one rank),
+ * col_offset < 0, ld_x < num_features, or a NULL d_gathered / d_out.            */
 int gp_decode_gathered(const uint64_t *d_gathered, int64_t rank_stride_words, int32_t num_ranks,
                        int64_t num_nodes, int64_t anchors_per_rank, int32_t num_planes,
                        int32_t batches, int32_t words_per_batch, int64_t plane_stride_words,

@@ -448,8 +448,20 @@ def test_peer_decode_variants_on_one_gpu(dev, k, f):
             assert torch.equal(out[:, f + r * k: f + (r + 1) * k], want[:, f:]), (ranks, r)
 
 
-@pytest.mark.parametrize("world,k,f", [(2, 64, 20), (4, 512, 500), (3, 48, 8), (8, 128, 4)])
-def test_push_exchange_virtual_ranks_on_one_gpu(dev, monkeypatch, world, k, f):
+@pytest.mark.parametrize("world,k,f,n,ldx", [
+    pytest.param(2, 64, 20, 3000, 20, id="2-64-20"),
+    pytest.param(4, 512, 500, 3000, 500, id="4-512-500"),
+    pytest.param(3, 48, 8, 3000, 8, id="3-48-8"),
+    pytest.param(8, 128, 4, 3000, 4, id="8-128-4"),
+    (2, 512, 20, 3000, 20),     # 256 lanes per rank: 4 words per batch, the benchmark's shard
+    (4, 1024, 4, 3000, 4),
+    (3, 984, 8, 3000, 8),       # 328 lanes: 2 batches, the last one ragged
+    (2, 1040, 12, 3000, 12),    # 520 lanes: 3 batches
+    (2, 1040, 12, 3001, 12),    # and N not a multiple of the row block
+    (2, 64, 20, 3001, 20),      # 8-byte rows, odd N: the last block's segment is rounded up to 16 bytes
+    (4, 128, 20, 3000, 21),     # x a column slice with a pitch that is not a multiple of 4: scalar x copy
+])
+def test_push_exchange_virtual_ranks_on_one_gpu(dev, monkeypatch, world, k, f, n, ldx):
     """gp_exchange.cu with `world` virtual ranks in ONE process on one GPU (plain device pointers instead of IPC
     mappings): every rank runs its anchor shard, then the fused pack / push / decode kernels run side by side on
     their own streams (partial grids so all of them are resident) and every rank's [N, F + K] matrix must equal the
@@ -458,12 +470,11 @@ def test_push_exchange_virtual_ranks_on_one_gpu(dev, monkeypatch, world, k, f):
 
     from graphpope_b200 import _lib, distributed as gpd
     lib = _lib.load()
-    n = 3000
     ei = synth.chung_lu_symmetric(n, 18000, 2.2, seed=5)
     ei = np.concatenate([ei, synth.random_digraph(n, 700, seed=6)], axis=1)
     per = k // world
     ei_d = torch.as_tensor(ei).cuda()
-    x = torch.randn(n, f, device="cuda")
+    x = torch.randn(n, ldx, device="cuda")[:, :f]
     engines = [dev.GeodesicEngine(n, ei.shape[1], per) for _ in range(world)]
     xch = [gpd.PushExchange(engines[r], world=world, rank=r, grid_blocks=24) for r in range(world)]
     for r in range(world):
@@ -482,7 +493,7 @@ def test_push_exchange_virtual_ranks_on_one_gpu(dev, monkeypatch, world, k, f):
         torch.cuda.synchronize()
         for r in range(world):
             with torch.cuda.stream(streams[r]):
-                _lib.check(lib.gp_exchange_run(xch[r]._h, c_void_p(x.data_ptr()), f, f, c_void_p(outs[r].data_ptr()),
+                _lib.check(lib.gp_exchange_run(xch[r]._h, c_void_p(x.data_ptr()), f, ldx, c_void_p(outs[r].data_ptr()),
                                                f + k, f, c_void_p(streams[r].cuda_stream)))
         torch.cuda.synchronize()
         for r in range(world):
