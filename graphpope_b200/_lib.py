@@ -82,18 +82,19 @@ SIGNATURES = {
                                 POINTER(c_int32), POINTER(c_int32), c_void_p]),
     "gp_decode_gathered": (c_int, [c_void_p, c_int64, c_int32, c_int64, c_int64, c_int32, c_int32, c_int32,
                                    c_int64, c_void_p, c_int64, c_int64, c_void_p, c_int64, c_int64, c_void_p]),
+    # round 1's pull exchange, removed: these five return GP_ERR_UNSUPPORTED (kept for ABI version 1)
     "gp_msbfs_pack": (c_int, [c_void_p, c_int32, POINTER(c_void_p), POINTER(c_int64), POINTER(c_int32),
                               POINTER(c_int32), POINTER(c_void_p), c_void_p]),
     "gp_geodesic_run_packed": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int32, c_void_p]),
     "gp_msbfs_packed_info": (c_int, [c_void_p, c_int32, POINTER(c_void_p), POINTER(c_int64), POINTER(c_int32),
                                      POINTER(c_int32), POINTER(c_void_p)]),
     "gp_msbfs_ipc_export": (c_int, [c_void_p, c_void_p, POINTER(c_int64)]),
-    "gp_ipc_open": (c_int, [c_void_p, POINTER(c_void_p)]),
-    "gp_ipc_close": (c_int, [c_void_p]),
     "gp_decode_peers": (c_int, [c_void_p, c_int32, c_int64, c_int64, c_int32, c_int32, c_int64, c_void_p, c_int64,
                                 c_int64, c_void_p, c_int64, c_int64, c_void_p]),
     "gp_exchange_create": (c_int, [c_void_p, c_int32, c_int32, POINTER(c_void_p)]),
     "gp_exchange_ipc_export": (c_int, [c_void_p, c_void_p]),
+    "gp_ipc_open": (c_int, [c_void_p, POINTER(c_void_p)]),
+    "gp_ipc_close": (c_int, [c_void_p]),
     "gp_exchange_local_ptr": (c_int, [c_void_p, POINTER(c_void_p)]),
     "gp_exchange_set_peer": (c_int, [c_void_p, c_int32, c_void_p]),
     "gp_geodesic_run_exchange": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p,

@@ -412,8 +412,7 @@ int run_pipeline_eager(gp_csr *csr, gp_msbfs *bfs, const int64_t *d_ei, int64_t 
     }
     GpRange r(xchg != nullptr ? "graphpope:exchange_decode" : "graphpope:epilogue");
     if (xchg != nullptr) GP_TRY(gp_exchange_launch(xchg, parity, d_x, f, ldx, d_out, ldo, coff, s));
-    else if (d_out != nullptr) GP_TRY(gp_msbfs_features(bfs, d_x, f, ldx, d_out, ldo, coff, s));
-    else GP_TRY(gp_msbfs_pack(bfs, (int32_t)coff, nullptr, nullptr, nullptr, nullptr, nullptr, s));  // coff = slot
+    else if (d_out != nullptr) GP_TRY(gp_msbfs_features(bfs, d_x, f, ldx, d_out, ldo, coff, s));  // NULL: empty output
     if (stage_events) GP_CUDA_CHECK(cudaEventRecordWithFlags(bfs->ev_pipe1, s, ev_flags));
     bfs->pipe_timed = stage_events;
     return GP_OK;
@@ -514,6 +513,10 @@ extern "C" int gp_geodesic_run(gp_csr_t *csr, gp_msbfs_t *bfs, const int64_t *d_
                                int64_t num_features, int64_t ld_x, float *d_out, int64_t ld_out,
                                int64_t col_offset, gp_stream_t stream_)
 {
+    GP_REQUIRE(csr != nullptr && bfs != nullptr, GP_ERR_INVALID, "gp_geodesic_run: NULL handle");
+    // an empty [N, F+K] tensor may have no storage, so d_out may be NULL only when there is nothing to write
+    const bool writes = csr->num_nodes > 0 && (num_anchors > 0 || (d_x != nullptr && num_features > 0));
+    GP_REQUIRE(d_out != nullptr || !writes, GP_ERR_INVALID, "gp_geodesic_run: d_out is NULL");
     return geodesic_run_impl(csr, bfs, d_edge_index, num_edges, d_anchors, num_anchors, d_x, num_features, ld_x, d_out,
                              ld_out, col_offset, stream_, nullptr, 0);
 }
@@ -547,13 +550,12 @@ extern "C" int gp_concat_x(const float *d_x, int64_t num_nodes, int64_t num_feat
     return GP_OK;
 }
 
-// Sharded form: csr build + ms-bfs + pack into exchange slot `slot` (graph-replayed like gp_geodesic_run).
-extern "C" int gp_geodesic_run_packed(gp_csr_t *csr, gp_msbfs_t *bfs, const int64_t *d_edge_index, int64_t num_edges,
-                                      const int64_t *d_anchors, int64_t num_anchors, int32_t slot, gp_stream_t stream)
+// Round 1's pull exchange was removed (its other four entry points are in gp_epilogue.cu); kept so that programs
+// built against ABI version 1 still link.
+extern "C" int gp_geodesic_run_packed(gp_csr_t *, gp_msbfs_t *, const int64_t *, int64_t, const int64_t *, int64_t,
+                                      int32_t, gp_stream_t)
 {
-    GP_REQUIRE(slot == 0 || slot == 1, GP_ERR_INVALID, "gp_geodesic_run_packed: slot must be 0 or 1");
-    return gp_geodesic_run(csr, bfs, d_edge_index, num_edges, d_anchors, num_anchors, nullptr, 0, 0, nullptr, 0, slot,
-                           stream);
+    GP_REQUIRE(false, GP_ERR_UNSUPPORTED, "gp_geodesic_run_packed: removed, use gp_geodesic_run_exchange");
 }
 
 extern "C" int gp_host_concat(const float *h_x, int64_t num_features, const float *h_block, int64_t block_cols,

@@ -27,6 +27,7 @@
 // peer memory back-pressure the SM's local streaming stores (phase times 1.3-2x), a fence.sc.sys before the flag
 // costs ~20 us behind them, dedicated pushing blocks need dynamic row hand-out whose same-address atomics cost
 // ~30 us per pass.
+#include "gp_epilogue.cuh"
 #include "gp_msbfs.cuh"
 #include "gp_tma.cuh"
 
@@ -56,6 +57,7 @@ constexpr size_t XCHG_FLAG_BYTES = 256;
 constexpr int XCHG_STAGES = 3;
 constexpr int XCHG_STAGE_CAP = 18 * 1024;  // bytes of peer segments per stage
 constexpr long long GP_XCHG_TIMEOUT_CYCLES = 16000000000ll;  // ~8 s at 1.9 GHz
+constexpr int GP_PACKED_ARRAYS = 5;  // exchange format: reached mask + 4 hop-index bit planes
 
 struct XchgParams {
     // local result (gp_msbfs.cu layout)
@@ -79,8 +81,6 @@ struct XchgParams {
     int vec_x;
 };
 
-__device__ __forceinline__ float inv_hops_x(u32 d) { return __fdiv_rn(1.0f, __uint2float_rn(d + 1u)); }
-
 __device__ __forceinline__ u64 *packed_ptr(const XchgParams &p, int rank)
 {
     return reinterpret_cast<u64 *>(p.peer[rank] + XCHG_FLAG_BYTES) + (size_t)p.parity * GP_PACKED_ARRAYS * p.pk_stride;
@@ -89,32 +89,6 @@ __device__ __forceinline__ u64 *packed_ptr(const XchgParams &p, int rank)
 __device__ __forceinline__ u32 *flag_ptr(const XchgParams &p, int dest, int src)
 {
     return reinterpret_cast<u32 *>(p.peer[dest]) + p.parity * GP_MAX_RANKS + src;
-}
-
-__device__ __forceinline__ void copy_x_row_x(const float *xrow, float *orow, int f, int lane, int vec_x)
-{
-    constexpr int T = 4;
-    if (vec_x) {
-        const float4 *x4 = reinterpret_cast<const float4 *>(xrow);
-        float4 *o4 = reinterpret_cast<float4 *>(orow);
-        const int q = f >> 2;
-        for (int i0 = 0; i0 < q; i0 += 32 * T) {
-            float4 v[T];
-#pragma unroll
-            for (int t = 0; t < T; ++t) {
-                const int i = i0 + lane + 32 * t;
-                if (i < q) v[t] = __ldcs(x4 + i);
-            }
-#pragma unroll
-            for (int t = 0; t < T; ++t) {
-                const int i = i0 + lane + 32 * t;
-                if (i < q) __stcs(o4 + i, v[t]);
-            }
-        }
-        for (int i = (q << 2) + lane; i < f; i += 32) orow[i] = __ldcs(xrow + i);
-    } else {
-        for (int i = lane; i < f; i += 32) orow[i] = __ldcs(xrow + i);
-    }
 }
 
 // 8 columns of one (node, rank, batch, lane byte) from the 5 packed bytes.
@@ -137,7 +111,7 @@ __global__ void __launch_bounds__(XCHG_THREADS, 4) exchange_decode_kernel(XchgPa
     __shared__ float s_inv[16];
     __shared__ u32 s_epoch;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    if (tid < 16) s_inv[tid] = inv_hops_x((u32)tid);
+    if (tid < 16) s_inv[tid] = inv_hops((u32)tid);
     if (tid == 0) {
         // The epoch of this step: one more than the rank's counter for this parity.  The counter is bumped by the
         // last block to LEAVE the kernel, i.e. after every block has read it here.
@@ -263,7 +237,7 @@ __global__ void __launch_bounds__(XCHG_THREADS, 4) exchange_decode_kernel(XchgPa
         const unsigned char *st = s_stage + (size_t)s * p.stage_bytes;
         for (long long u = u0 + warp; u < u1; u += XCHG_WARPS) {
             float *orow = p.out + (size_t)u * p.ld_out;
-            if (p.x != nullptr) copy_x_row_x(p.x + (size_t)u * p.ld_x, orow, (int)p.num_features, lane, p.vec_x);
+            if (p.x != nullptr) copy_x_row(p.x + (size_t)u * p.ld_x, orow, (int)p.num_features, lane, p.vec_x);
             for (int b = 0; b < p.batches; ++b) {
                 const int col0 = b * 64 * p.wb + lane * 8;
                 if (lane >= row_bytes || col0 >= p.kr) continue;
@@ -347,6 +321,21 @@ extern "C" int gp_exchange_ipc_export(gp_exchange_t *x, uint8_t *handle64)
     cudaIpcMemHandle_t hd;
     GP_CUDA_CHECK(cudaIpcGetMemHandle(&hd, x->buf));
     memcpy(handle64, &hd, 64);
+    return GP_OK;
+}
+
+extern "C" int gp_ipc_open(const uint8_t *handle64, void **d_ptr)
+{
+    GP_REQUIRE(handle64 != nullptr && d_ptr != nullptr, GP_ERR_INVALID, "gp_ipc_open: NULL argument");
+    cudaIpcMemHandle_t hd;
+    memcpy(&hd, handle64, 64);
+    GP_CUDA_CHECK(cudaIpcOpenMemHandle(d_ptr, hd, cudaIpcMemLazyEnablePeerAccess));
+    return GP_OK;
+}
+
+extern "C" int gp_ipc_close(void *d_ptr)
+{
+    if (d_ptr) GP_CUDA_CHECK(cudaIpcCloseMemHandle(d_ptr));
     return GP_OK;
 }
 

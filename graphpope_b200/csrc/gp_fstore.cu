@@ -15,7 +15,7 @@ namespace {
 constexpr int FS_MAX_PLANES = 1 + GP_BFS_PLANES;  // 17: hops up to 65534
 
 // One thread per (node, lane word).  Hop bits 0..3 are ORs of the level arrays R[1..levels], as in
-// pack_result_kernel; lanes first reached at hop >= 16 carry their whole hop count in the deep planes R[16 + q] and
+// the exchange's pack (gp_exchange.cu); lanes first reached at hop >= 16 carry their whole hop count in the deep planes R[16 + q] and
 // have zeros in R[1..15], so the two sources are disjoint.
 __global__ void __launch_bounds__(256) fstore_pack_kernel(const u64 *__restrict__ result, long long plane_stride,
                                                           long long n, int wb, int words, int levels, int deep,

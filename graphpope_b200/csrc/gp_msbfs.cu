@@ -723,8 +723,6 @@ extern "C" int gp_msbfs_free(gp_msbfs_t *h)
     cudaFree(h->scratch);  // the lane arrays live in the same allocation
     cudaFree(h->hub_acc);
     cudaFree(h->hub_cnt);
-    cudaFree(h->packed);
-    cudaFree(h->deep_flag);
     cudaFree(h->trace);
     if (h->ev_start) cudaEventDestroy(h->ev_start);
     if (h->ev_stop) cudaEventDestroy(h->ev_stop);

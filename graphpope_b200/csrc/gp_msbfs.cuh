@@ -54,8 +54,6 @@ struct gp_msbfs {
     int map_want_bytes = -1; // map size the cached launch configuration was computed for
     int64_t hub_capacity = 0;
     bool hub_zeroed = false;
-    u64 *packed = nullptr;   // [2 slots][GP_PACKED_ARRAYS][cap words] exchange buffers (allocated on first pack)
-    int *deep_flag = nullptr;  // device int: 1 if the last packed run had hops > 15 (packed format invalid)
     int *status = nullptr;      // [GP_BFS_ST_WORDS]
     u64 *counters = nullptr;    // [4] gathers issued, unused, %globaltimer at kernel entry and after the last level
     u64 *trace = nullptr;       // [32 levels][warps][4] phase clocks, only with GP_BFS_TRACE=1
@@ -73,7 +71,9 @@ void gp_msbfs_layout(gp_msbfs *h, int64_t num_anchors);
 // stream capture only on request (an event-record NODE costs ~4 us of the replayed step: 246 -> 231 us without the four).
 bool gp_stage_events_on(const gp_msbfs *h);
 
-// Fused decode + concat epilogue over `num_ranks` plane sets (1 = local result).
+// Fused decode + concat epilogue over `num_ranks` plane sets (1 = local result).  The decode kernels take it as a
+// __grid_constant__ parameter and read its fields in place: copied into registers up front, they push
+// decode_features_bytes_kernel, which sits at its 64-register bound, into spills.
 struct GpDecodeParams {
     const u64 *planes0;        // result block of rank 0 (R[0..], gp_msbfs.cu), R[0] = reached mask
     long long rank_stride;     // words between consecutive ranks' result blocks
@@ -88,10 +88,5 @@ struct GpDecodeParams {
     long long num_features, ld_x;
     float *out;
     long long ld_out, col_offset;
-    // packed exchange format (gp_msbfs_pack): 5 arrays per rank = reached mask + 4 hop-index bit planes,
-    // read in place from every rank's buffer (own memory or NVLink peer mappings)
-    int packed;
-    const u64 *rank_ptr[GP_MAX_RANKS];
 };
-constexpr int GP_PACKED_ARRAYS = 5;
 int gp_launch_decode_features(const GpDecodeParams &p, cudaStream_t stream);

@@ -3,9 +3,11 @@
 The reference shards its CPU pool by *node slice* (utils.py:99-100) because its unit of work is
 a (node, anchor) pair; every DDP rank then recomputes the identical embedding (main.py:88-98).
 Here the BFS is sharded by *anchor*: the CSR is replicated, rank r owns anchors
-``[r*K/G, (r+1)*K/G)`` as its own bit lanes, and there is no exchange during traversal.  The one
-real exchange step is assembling the replicated ``[N, F+K]`` output: ranks all-gather their
-bit-sliced result planes (≈ (1 + log2(max hops)) bits per (node, anchor) instead of 16 or 32) and
+``[r*K/G, (r+1)*K/G)`` as its own bit lanes, and there is no exchange during traversal.  The
+exchange step assembles the replicated ``[N, F+K]`` output.  :class:`PushExchange` does it in one
+kernel over NVLink peer memory, in a 5-plane format that holds hops up to 15.  When a shard has
+deeper hops, :func:`sharded_geodesic_features` is the fallback: ranks all-gather their bit-sliced
+result planes (≈ (1 + log2(max hops)) bits per (node, anchor) instead of 16 or 32) over NCCL and
 each rank's epilogue kernel decodes all shards, performing the ``[G][N][K/G] -> [N, F + g*K/G + j]``
 column permutation while it writes fp32.
 
@@ -209,7 +211,7 @@ def sharded_geodesic_features(engine, edge_index: torch.Tensor, anchors: torch.T
         return engine.run(edge_index, anchors, x, out)
     if k % world:
         raise ValueError(f"the all-gather path needs num_anchor_nodes={k} divisible by the world size {world}; "
-                         "PeerAssembly pads a ragged K itself")
+                         "PushExchange pads a ragged K itself")
     lo, hi = shard_bounds(k, world, rank)
     engine.csr.build(edge_index)
     engine.bfs.run(anchors[lo:hi].contiguous())
@@ -225,56 +227,6 @@ def sharded_geodesic_features(engine, edge_index: torch.Tensor, anchors: torch.T
                                  meta["batches"], meta["words_per_batch"], stride, _ptr(x), f,
                                  x.stride(0) if x is not None and n > 1 else f, _ptr(out),
                                  out.stride(0) if n > 1 else f + k, f, _stream()))
-    return out
-
-
-def sharded_geodesic_embed_host(engine, edge_index: torch.Tensor, anchors, x: torch.Tensor | None,
-                                out: torch.Tensor, staging: dict, group=None, peer=None) -> torch.Tensor:
-    """Host-buffer form of the sharded path (what a DataModule calls): HOST ``edge_index`` / ``x`` in,
-    HOST float32 ``[N, F + K]`` out.  ``staging`` caches the device / pinned scratch between calls."""
-    from . import _lib
-    from ._lib import check
-    from .device import _ptr
-
-    n = engine.csr.num_nodes
-    a = torch.as_tensor(anchors)
-    k = a.numel()
-    f = 0 if x is None else x.size(1)
-    if staging.get("shape") != (n, k, edge_index.size(1)):
-        staging.clear()
-        staging["shape"] = (n, k, edge_index.size(1))
-        staging["ei"] = torch.empty_like(edge_index, device="cuda")
-        staging["anchors"] = torch.empty(k, dtype=torch.int64, device="cuda")
-        staging["block_d"] = torch.empty((n, k), dtype=torch.float32, device="cuda")
-        staging["block_h"] = torch.empty((n, k), dtype=torch.float32).pin_memory()
-    staging["ei"].copy_(edge_index, non_blocking=True)
-    staging["anchors"].copy_(a, non_blocking=True)
-    lib = _lib.load()
-    direct = out.is_pinned() and out.stride(1) == 1  # strided DMA straight into columns [F, F + K) of `out`
-
-    def device_to_host():
-        if direct:
-            check(lib.gp_block_to_host(_ptr(staging["block_d"]), n, k, _ptr(out), out.stride(0), f,
-                                       c_void_p(torch.cuda.current_stream().cuda_stream)))
-        else:
-            staging["block_h"].copy_(staging["block_d"], non_blocking=True)  # one contiguous DMA, scattered below
-
-    if peer is not None:
-        _, deep = peer.run(staging["ei"], staging["anchors"], None, staging["block_d"])
-    else:
-        deep = None
-        sharded_geodesic_features(engine, staging["ei"], staging["anchors"], None, staging["block_d"], group)
-    device_to_host()
-    # concat_into_features (utils.py:129-135): x goes into columns [0, F) on the host while the GPU works
-    if x is not None:
-        check(lib.gp_host_concat(_ptr(x), f, None, 0, n, _ptr(out), out.stride(0)))
-    torch.cuda.current_stream().synchronize()
-    if deep is not None and int(deep.item()) != 0:  # hops > 15 somewhere: redo through the all-gather path
-        sharded_geodesic_features(engine, staging["ei"], staging["anchors"], None, staging["block_d"], group)
-        device_to_host()
-        torch.cuda.current_stream().synchronize()
-    if not direct:
-        check(lib.gp_host_concat(None, f, _ptr(staging["block_h"]), k, n, _ptr(out), out.stride(0)))
     return out
 
 
@@ -368,8 +320,8 @@ def sharded_embed_host_shared(engine, edge_index: torch.Tensor, anchors, x: torc
     Rank r runs the MS-BFS for its anchor shard only, decodes its own ``[N, K/G]`` block and DMAs it straight
     into columns ``[F + lo, F + hi)`` of the shared matrix; the copy of ``x`` (concat_into_features,
     utils.py:129-135) is split by row range across the ranks; one barrier, then every rank returns the same
-    tensor.  Per rank and step: H2D = edge_index + its anchors, D2H = N * K/G floats (1/G of what the
-    replicated assembly moved), host copy = N/G rows of x.  Bit-equal to the 1-GPU result.
+    tensor.  Per rank and step: H2D = edge_index + its anchors, D2H = N * K/G floats (1/G of the anchor
+    block), host copy = N/G rows of x.  Bit-equal to the 1-GPU result.
     """
     from . import _lib
     from ._lib import check
@@ -520,7 +472,7 @@ class PushExchange:
         check(self.lib.gp_exchange_status(self._h, ctypes.byref(deep), _stream()))
         return int(deep.value)
 
-    trace_events = ()
+    trace_events = ()  # no host-side phase events per step; bench.py reads the attribute
 
     def trace(self):
         """Diagnostics: microseconds from the start of the last exchange kernel (block 0) to: its share packed, every
@@ -548,129 +500,5 @@ class PushExchange:
             pass
 
 
-def PeerAssembly(engine, group=None):
-    """The device exchange of the sharded path: the push kernel (default) or round 1's pull-based peer decode
-    (``GP_EXCHANGE=pull``: pack + NCCL flag all-reduce + an epilogue that reads the peers' shards over NVLink)."""
-    if os.environ.get("GP_EXCHANGE", "push") == "pull":
-        return PullAssembly(engine, group)
-    return PushExchange(engine, group)
-
-
-class PullAssembly:
-    """NVLink peer-to-peer assembly of the sharded result (the B200-native form of the exchange step).
-
-    Instead of all-gathering result masks into a staging buffer and then decoding, every rank maps the
-    other ranks' packed result buffers (CUDA IPC over NVSwitch) once, and the fused epilogue kernel
-    reads them *in place* while it writes the fp32 rows: own shard from HBM, peer shards through
-    NVLink loads, so the transfer overlaps the HBM-bound output writes tile by tile.  Per step there
-    is one tiny NCCL all-reduce (it carries the "hops > 15" flag and doubles as the cross-GPU barrier
-    that orders pack before decode); buffers are double-buffered so no second barrier is needed.
-    """
-
-    def __init__(self, engine, group=None):
-        import ctypes
-
-        from . import _lib
-        from ._lib import check
-
-        self.engine, self.group = engine, group
-        self.world = dist.get_world_size(group)
-        self.rank = dist.get_rank(group)
-        if self.world > 8:
-            raise ValueError("PeerAssembly covers the GPUs of one NVSwitch node (<= 8 ranks)")
-        self.lib = _lib.load()
-        handle = (ctypes.c_uint8 * 64)()
-        slot_stride = ctypes.c_int64()
-        check(self.lib.gp_msbfs_ipc_export(engine.bfs._h, handle, ctypes.byref(slot_stride)))
-        self.slot_stride_words = slot_stride.value
-        mine = torch.tensor(list(bytes(handle)), dtype=torch.uint8, device="cuda")
-        every = torch.empty(self.world * 64, dtype=torch.uint8, device="cuda")
-        dist.all_gather_into_tensor(every, mine, group=group)
-        every = every.cpu().view(self.world, 64)
-        self.base = []
-        self._opened = []
-        for r in range(self.world):
-            if r == self.rank:
-                self.base.append(None)  # filled from gp_msbfs_pack (own allocation)
-                continue
-            buf = (ctypes.c_uint8 * 64)(*every[r].tolist())
-            ptr = ctypes.c_void_p()
-            check(self.lib.gp_ipc_open(buf, ctypes.byref(ptr)))
-            self.base.append(ptr.value)
-            self._opened.append(ptr.value)
-        self.step = 0
-        self.trace_events = []
-        self.flag = torch.zeros(1, dtype=torch.int32, device="cuda")
-
-    def close(self):
-        for p in self._opened:
-            self.lib.gp_ipc_close(c_void_p(p))
-        self._opened = []
-
-    def run(self, edge_index, anchors, x=None, out=None):
-        """Same contract as :func:`sharded_geodesic_features`; returns (out, deep) where ``deep`` is a
-        device int32 that is 1 if some shard had hops > 15 (then the caller must use the gather path)."""
-        import ctypes
-
-        from ._lib import check
-        from .device import _ptr, _stream
-
-        eng = self.engine
-        n = eng.csr.num_nodes
-        k = anchors.numel()
-        f = 0 if x is None else x.size(1)
-        if out is None:
-            out = torch.empty((n, f + k), dtype=torch.float32, device="cuda")
-        lo, hi = shard_bounds(k, self.world, self.rank)
-        slot = self.step & 1
-        self.step += 1
-        key = (anchors.data_ptr(), lo, hi)
-        if getattr(self, "_shard_key", None) != key:  # keep the shard tensor alive and its pointer stable (graph key)
-            self._shard_key, self._shard = key, anchors[lo:hi].contiguous()
-        edge_index = edge_index.contiguous()
-        eng.csr._edges, eng.bfs._anchors, eng.bfs.num_anchors = edge_index, self._shard, hi - lo
-        trace = os.environ.get("GP_PEER_TRACE") is not None  # diagnostics: device time of the three phases
-        if trace:
-            ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
-            ev[0].record()
-        check(self.lib.gp_geodesic_run_packed(eng.csr._h, eng.bfs._h, _ptr(edge_index), edge_index.size(1),
-                                              _ptr(self._shard), hi - lo, slot, _stream()))
-        if trace:
-            ev[1].record()
-        packed, stride = ctypes.c_void_p(), ctypes.c_int64()
-        batches, wb, deep = ctypes.c_int32(), ctypes.c_int32(), ctypes.c_void_p()
-        check(self.lib.gp_msbfs_packed_info(eng.bfs._h, slot, ctypes.byref(packed), ctypes.byref(stride),
-                                            ctypes.byref(batches), ctypes.byref(wb), ctypes.byref(deep)))
-        # flag <- max over ranks of "my shard is deep"; stream-ordered, so it is also the barrier between
-        # every rank's pack and every rank's decode
-        self.flag.copy_(_wrap_device_words_i32(deep.value), non_blocking=True)
-        dist.all_reduce(self.flag, op=dist.ReduceOp.MAX, group=self.group)
-        if trace:
-            ev[2].record()
-        ptrs = (ctypes.c_void_p * self.world)()
-        for r in range(self.world):
-            base = packed.value - slot * self.slot_stride_words * 8 if r == self.rank else self.base[r]
-            ptrs[r] = base + slot * self.slot_stride_words * 8
-        check(self.lib.gp_decode_peers(ptrs, self.world, n, hi - lo, batches.value, wb.value, stride.value, _ptr(x), f,
-                                       x.stride(0) if x is not None and n > 1 else f, _ptr(out),
-                                       out.stride(0) if n > 1 else f + k, f, _stream()))
-        if trace:
-            ev[3].record()
-            self.trace_events.append(ev)
-        return out, self.flag
-
-    def trace_summary(self):
-        """Median device milliseconds of (csr + bfs + pack, flag all-reduce, peer decode) over the traced steps."""
-        import statistics
-        torch.cuda.synchronize()
-        cols = [[e[i].elapsed_time(e[i + 1]) for e in self.trace_events] for i in range(3)]
-        return [statistics.median(c) for c in cols] if self.trace_events else None
-
-
-def _wrap_device_words_i32(ptr: int) -> torch.Tensor:
-    class _Holder:
-        pass
-
-    h = _Holder()
-    h.__cuda_array_interface__ = {"shape": (1,), "typestr": "<i4", "data": (ptr, False), "version": 2}
-    return torch.as_tensor(h, device="cuda")
+# The name bench.py, tools/dist_check.py and INTEGRATION.md use for the device exchange.
+PeerAssembly = PushExchange

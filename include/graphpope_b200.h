@@ -147,7 +147,9 @@ int gp_msbfs_trace(gp_msbfs_t *bfs, uint64_t *h_out, int64_t cap_words, int32_t 
 int gp_msbfs_free(gp_msbfs_t *bfs);
 
 /* async.  gp_csr_build + gp_msbfs_run + gp_msbfs_features as ONE call.  Repeated calls with the same
- * arguments replay a captured CUDA graph (one launch instead of ~25); GP_USE_GRAPH=0 disables it.  */
+ * arguments replay a captured CUDA graph (one launch instead of ~25); GP_USE_GRAPH=0 disables it.
+ * GP_ERR_INVALID, before any launch, for a NULL d_out when the output has elements (N > 0 and K + F > 0;
+ * an empty output may be NULL).                                                                      */
 int gp_geodesic_run(gp_csr_t *csr, gp_msbfs_t *bfs, const int64_t *d_edge_index, int64_t num_edges,
                     const int64_t *d_anchors, int64_t num_anchors, const float *d_x, int64_t num_features,
                     int64_t ld_x, float *d_out, int64_t ld_out, int64_t col_offset, gp_stream_t stream);
@@ -156,8 +158,8 @@ int gp_geodesic_run(gp_csr_t *csr, gp_msbfs_t *bfs, const int64_t *d_edge_index,
  * Inside the captured pipeline of gp_geodesic_run an event-record NODE costs ~4 us of the replayed step (246 -> 231 us
  * for the four at Flickr size), so they are recorded only on request: gp_msbfs_set_stage_events(bfs, 1) (the handle's
  * captured pipelines are dropped and re-captured).  gp_pipeline_stage_ms (syncs on its own events): ms3[0] = csr build
- * (+ the MS-BFS state memset), ms3[1] = the persistent MS-BFS kernel, ms3[2] = epilogue (decode + concat, pack, or
- * the exchange kernel) of the last fused run.  gp_msbfs_kernel_device_ns needs no events: the kernel stamps
+ * (+ the MS-BFS state memset), ms3[1] = the persistent MS-BFS kernel, ms3[2] = epilogue (decode + concat, or the
+ * exchange kernel) of the last fused run.  gp_msbfs_kernel_device_ns needs no events: the kernel stamps
  * %globaltimer at its entry and after its last level.                                                        */
 int gp_msbfs_set_stage_events(gp_msbfs_t *bfs, int32_t enable);
 int gp_msbfs_kernel_device_ns(gp_msbfs_t *bfs, uint64_t *ns, gp_stream_t stream);
@@ -165,7 +167,7 @@ int gp_pipeline_stage_ms(gp_msbfs_t *bfs, float *ms3);
 
 /* async.  The x half of concat_into_features (utils.py:133-134) alone: d_out[:, 0:F] = d_x (a bulk-copy kernel for
  * 16-byte aligned rows, else one strided device-to-device transfer), for callers that want the copy on their own
- * stream; follow with gp_msbfs_features / gp_decode_peers called with d_x == NULL.  gp_geodesic_run keeps the copy
+ * stream; follow with gp_msbfs_features / gp_decode_gathered called with d_x == NULL.  gp_geodesic_run keeps the copy
  * inside its epilogue kernel: running it beside the csr build and the MS-BFS measured slower on B200 (copy engine
  * 0.323 ms, copy kernels 0.265-0.301 ms, against 0.246 ms per step).                                           */
 int gp_concat_x(const float *d_x, int64_t num_nodes, int64_t num_features, int64_t ld_x, float *d_out,
@@ -196,24 +198,16 @@ int gp_decode_gathered(const uint64_t *d_gathered, int64_t rank_stride_words, in
                        const float *d_x, int64_t num_features, int64_t ld_x,
                        float *d_out, int64_t ld_out, int64_t col_offset, gp_stream_t stream);
 
-/* ---- peer-to-peer assembly (NVLink / NVSwitch): no staging buffer, no all-gather.
- * gp_msbfs_pack (async) rewrites the last result into the fixed-size exchange format (reached mask +
- * 4 hop-index bit planes, valid for hops <= 15; *d_deep_flag tells on the device if that failed) in one
- * of two slots; gp_msbfs_ipc_export / gp_ipc_open hand the buffer to the other ranks of the node as CUDA
- * IPC mappings; gp_decode_peers (async) is the fused epilogue whose loads read every rank's buffer in
- * place — its own from HBM, the peers' over NVLink — while it writes the [N, F+K] rows.               */
+/* ---- removed: round 1's peer-to-peer assembly (pack into slots, decode reading the peers' slots in place).
+ * These five stay exported for programs built against ABI version 1; each returns GP_ERR_UNSUPPORTED before
+ * any CUDA call.  Use gp_geodesic_run_exchange.                                                            */
 int gp_msbfs_pack(gp_msbfs_t *bfs, int32_t slot, const uint64_t **d_packed, int64_t *plane_stride_words,
                   int32_t *batches, int32_t *words_per_batch, const int32_t **d_deep_flag, gp_stream_t stream);
-/* async.  gp_csr_build + gp_msbfs_run + gp_msbfs_pack(slot) as one graph-replayed call (a rank's share of
- * a sharded step up to the exchange).                                                                */
 int gp_geodesic_run_packed(gp_csr_t *csr, gp_msbfs_t *bfs, const int64_t *d_edge_index, int64_t num_edges,
                            const int64_t *d_anchors, int64_t num_anchors, int32_t slot, gp_stream_t stream);
-/* Pointers / shape of exchange slot `slot` without launching anything. */
 int gp_msbfs_packed_info(gp_msbfs_t *bfs, int32_t slot, const uint64_t **d_packed, int64_t *plane_stride_words,
                          int32_t *batches, int32_t *words_per_batch, const int32_t **d_deep_flag);
 int gp_msbfs_ipc_export(gp_msbfs_t *bfs, uint8_t *handle64, int64_t *slot_stride_words);
-int gp_ipc_open(const uint8_t *handle64, void **d_ptr);
-int gp_ipc_close(void *d_ptr);
 int gp_decode_peers(const uint64_t *const *h_rank_ptrs, int32_t num_ranks, int64_t num_nodes,
                     int64_t anchors_per_rank, int32_t batches, int32_t words_per_batch, int64_t plane_stride_words,
                     const float *d_x, int64_t num_features, int64_t ld_x, float *d_out, int64_t ld_out,
@@ -238,6 +232,9 @@ int gp_decode_peers(const uint64_t *const *h_rank_ptrs, int32_t num_ranks, int64
  *                           GP_ERR_CUDA if a peer's flag never arrived (bounded wait, ~8 s).                   */
 int gp_exchange_create(gp_msbfs_t *bfs, int32_t world, int32_t rank, gp_exchange_t **out);
 int gp_exchange_ipc_export(gp_exchange_t *xchg, uint8_t *handle64);
+/* Map another rank's exchange buffer from its IPC handle / unmap it (CUDA IPC). */
+int gp_ipc_open(const uint8_t *handle64, void **d_ptr);
+int gp_ipc_close(void *d_ptr);
 int gp_exchange_local_ptr(gp_exchange_t *xchg, void **d_ptr);
 int gp_exchange_set_peer(gp_exchange_t *xchg, int32_t rank, void *d_ptr);
 int gp_geodesic_run_exchange(gp_csr_t *csr, gp_msbfs_t *bfs, gp_exchange_t *xchg, const int64_t *d_edge_index,

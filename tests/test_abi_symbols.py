@@ -53,6 +53,17 @@ def test_no_compute_without_gpu_but_clean_errors():
     assert lib.gp_eigenvector(None, 1e-15, 10, None, None, None) == _lib.GP_ERR_INVALID
     assert lib.gp_concat_x(None, 4, 4, 2, None, 8, None) == _lib.GP_ERR_INVALID  # ld_x < F
     assert lib.gp_concat_x(None, 0, 4, 4, None, 8, None) == _lib.GP_OK            # nothing to copy
+    # round 1's pull exchange: exported for ABI 1 callers, refused without touching the device
+    removed = {
+        "gp_msbfs_pack": (None, 0, None, None, None, None, None, None),
+        "gp_geodesic_run_packed": (None, None, None, 0, None, 0, 0, None),
+        "gp_msbfs_packed_info": (None, 0, None, None, None, None, None),
+        "gp_msbfs_ipc_export": (None, None, None),
+        "gp_decode_peers": (None, 0, 0, 0, 0, 0, 0, None, 0, 0, None, 0, 0, None),
+    }
+    for name, args in removed.items():
+        assert getattr(lib, name)(*args) == _lib.GP_ERR_UNSUPPORTED, name
+        assert lib.gp_last_error() == f"{name}: removed, use gp_geodesic_run_exchange".encode(), name
 
 
 def test_product_never_imports_the_oracle():

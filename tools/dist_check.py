@@ -33,7 +33,7 @@ for name, k_total in (("pubmed-shape", 256), ("flickr-shape", 1024), ("flickr-sh
     for _ in range(10): gpd.sharded_geodesic_features(eng, ei_d, a_d, x_d, out)
     ev1.record(); torch.cuda.synchronize()
     if rank == 0: print(f"    sharded step (NCCL all-gather of masks) {ev0.elapsed_time(ev1) / 10:.3f} ms", flush=True)
-    # peer-to-peer assembly: epilogue reads the other ranks' packed buffers over NVLink
+    # peer-to-peer assembly: one kernel packs this rank's shard and bulk-copies the peers' packed rows over NVLink
     peer = gpd.PeerAssembly(eng)
     out2, deep = peer.run(ei_d, a_d, x_d)
     torch.cuda.synchronize()
